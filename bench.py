@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native ray-traced lighting + SVGF chain.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one frame of the hybrid render path's hot chain on synthetic input:
     Raytrace Pass (shadow 1 spp + AO 1 spp per non-sky pixel)  ->  SVGF Denoise Pass (temporal + variance + 5 a-trous
@@ -387,6 +387,30 @@ class GpuFrameLoop:
         self.ctx.close()
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loop, rank, world):
+    """--dump-outputs: what the last timed step handed its caller, as float32 .npy files: the denoised shadow/AO image, the raw ray-traced
+    shadow/AO masks and, with reflections on, the reflection image ([H, W, C] each). Above the 64 MB budget (4K frames, or several ranks)
+    every array keeps the same seeded sample of pixels ([n, C], pixel indices ascending), so two builds can still be compared value for value."""
+    HP = loop.HP
+    k = loop.frame_no - 1
+    rt, refl = loop.path.rt_sets[(k & 1) if loop.fif == 2 else 0]
+    images = {"denoised_shadow_ao": HP.N_DENOISED, "raytraced_shadow_ao": rt}
+    if loop.refl:
+        images["raytraced_reflections"] = refl
+    arrays = {name: loop.ctx.image_download(img).astype(np.float32) for name, img in images.items()}
+    px = loop.W * loop.H
+    per_px = sum(a.nbytes for a in arrays.values()) // px
+    if per_px * px * world > DUMP_BUDGET_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(px, DUMP_BUDGET_BYTES // (per_px * world), replace=False))
+        arrays = {name: a.reshape(px, -1)[idx] for name, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 def timed(torch, stream, barrier, fn, n):
     """n calls of fn between two CUDA events on `stream`, barrier + synchronize on both sides. Returns (ms, sum of fn's return values)."""
     barrier()
@@ -695,7 +719,7 @@ def run_views64(args):
             ctx.bind_pass_images([g[HP.N_ALBEDO], g[HP.N_NORMALS], g[HP.N_MOTION], g[HP.N_DEPTH]])
             ctx.gbuffer_pass(W, H)
             rays_of[i] = int((ctx.image_download(g[HP.N_DEPTH]) > 0).sum()) * (1 + ao_spp + refl)
-        reps = max(1, args.steps // n_views) if args.steps >= n_views else 1
+        reps = args.steps // n_views
         sampler = ClockSampler(local)
         l0 = ctx.kernel_launches
         barrier(); sampler.start()
@@ -768,6 +792,8 @@ def run_gpu(args):
         ms_total, rays = timed(torch, stream, barrier, loop.step, K)
         clocks = sampler.stop()
         launches = ctx.kernel_launches - l0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, loop, rank, world)
         if fif == 2:
             # per-pass times need the passes one after the other: the same frames again, one frame in flight, with timestamps
             Kb = min(K, 50)
@@ -1068,7 +1094,15 @@ def main():
                     help="row-band mode: halo rows pushed by the kernels over NVLink peer memory (default) or NCCL send/recv between passes")
     ap.add_argument("--motion-halo", type=int, default=0,
                     help="rows of history/moments exchanged for the temporal pass (row-band mode); 0 = derive from the G-buffer's motion vectors")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the images the last one computed to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.workload.startswith("views64") and args.steps % 64:
+        ap.error("--workload views64_*: a step is one view and the views are timed in whole batches of 64, so --steps must be a multiple of 64")
+    if args.dump_outputs and (args.impl == "reference" or args.workload.startswith("views64") or args.partition == "rows"):
+        ap.error("--dump-outputs applies to the GPU frame loop (--impl b200, one view per rank)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
