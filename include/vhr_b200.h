@@ -344,6 +344,18 @@ int vhr_debug_download_reflection_t(vhr_context *ctx, float *host, size_t bytes)
  * 2 motion/metallic-roughness, 3 depth. */
 int vhr_gbuffer_pass(vhr_context *ctx, uint32_t width, uint32_t height);
 
+/* Shadow-map producer as a CUDA depth rasteriser (stand-in for the rasterised "Shadow Map Pass", hybrid_render_path.cpp:58-99,
+ * depth_prepass.vert/.frag). Bound image 0 is the Shadow Map: D32_SFLOAT, any size (4096 x 4096 in the reference's graph).
+ * Draws the world-space triangles of the last vhr_update_geometry, two-sided, through directional_light.projview of the
+ * per-frame constants; viewport without Y flip (row 0 = NDC y -1), vertices snapped to 1/256 texel, samples at texel centres
+ * with a top-left fill rule, depth kept where 0 <= z <= 1 and combined by max (reverse-Z, cleared to 0). DESIGN.md §2 states
+ * the exact arithmetic; the result does not depend on the order of the triangles. projview must be finite with a last row
+ * of (0, 0, 0, 1) (an orthographic light, as the scene loader builds) or all zero (a scene without a light: the map is only
+ * cleared); anything else is VHR_ERR_INVALID. VHR_ERR_STATE without geometry or per-frame constants; VHR_ERR_CUDA on a
+ * VHR_DEVICE_NONE context. VHR_OPT_ROW_BEGIN / END do not apply (the map is not display-sized), and under a partition every
+ * rank renders the whole map (replicated input, like the acceleration structure). Runs on the selected queue. */
+int vhr_shadow_map_pass(vhr_context *ctx);
+
 #ifdef __cplusplus
 }
 #endif

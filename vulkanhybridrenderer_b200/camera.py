@@ -71,6 +71,55 @@ def directional_light(direction, color=(1.0, 1.0, 1.0), intensity=30.0):
     return dl
 
 
+def _ortho_reverse_z(l, r, b, t, zn, zf):
+    """glm::orthoRH_ZO(l, r, b, t, zn, zf) (GLM_FORCE_DEPTH_ZERO_TO_ONE): with zn > zf, depth 0 at distance zn, 1 at zf."""
+    p = np.eye(4)
+    p[0, 0], p[1, 1], p[2, 2] = 2.0 / (r - l), 2.0 / (t - b), -1.0 / (zf - zn)
+    p[0, 3], p[1, 3], p[2, 3] = -(r + l) / (r - l), -(t + b) / (t - b), -zn / (zf - zn)
+    return p
+
+
+def _look_at(eye, center, up):
+    """glm::lookAtRH"""
+    f = np.asarray(center, np.float64) - eye
+    f = f / np.linalg.norm(f)
+    s = np.cross(f, up)
+    s = s / np.linalg.norm(s)
+    u = np.cross(s, f)
+    v = np.eye(4)
+    v[0, :3], v[1, :3], v[2, :3] = s, u, -f
+    v[0, 3], v[1, 3], v[2, 3] = -s @ eye, -u @ eye, f @ eye
+    return v
+
+
+def light_projview(direction):
+    """directional_light.projview as the reference's scene loader builds it (scene_loader.cpp:74-100, host/scene_loader.cpp
+    setup_directional_light): glm::ortho(-8, 8, -8, 8, 12, 0.1) * glm::lookAt(-12 d, 0, +y), column-major float32. The window is
+    fixed: depth 0 lies on the plane through the origin, so geometry farther from the light than the origin is clipped."""
+    d = np.asarray(direction, np.float64)[:3]
+    d = d / np.linalg.norm(d)
+    pv = _ortho_reverse_z(-8.0, 8.0, -8.0, 8.0, 12.0, 0.1) @ _look_at(-12.0 * d, np.zeros(3), np.array([0.0, 1.0, 0.0]))
+    return to_glm(pv)
+
+
+def fit_light_projview(direction, scene_min, scene_max, margin=0.01):
+    """Test and timing harness only (the reference has no such matrix): the same ortho * lookAt form, with a window and near / far
+    planes that enclose the box [scene_min, scene_max] seen along `direction` (plus `margin` of its diagonal), so that nothing is
+    clipped. Depth 1 is the nearest point of the box, 0 the farthest."""
+    d = np.asarray(direction, np.float64)[:3]
+    d = d / np.linalg.norm(d)
+    lo, hi = np.asarray(scene_min, np.float64), np.asarray(scene_max, np.float64)
+    c, r = 0.5 * (lo + hi), 0.5 * np.linalg.norm(hi - lo)
+    up = np.array([0.0, 1.0, 0.0]) if abs(d[1]) < 0.999 else np.array([0.0, 0.0, 1.0])
+    view = _look_at(c - d * (r + 1.0), c, up)
+    corners = np.array([[x, y, z, 1.0] for x in (lo[0], hi[0]) for y in (lo[1], hi[1]) for z in (lo[2], hi[2])]) @ view.T
+    pad = margin * 2.0 * r + 1e-6
+    (x0, y0), (x1, y1) = corners[:, :2].min(0) - pad, corners[:, :2].max(0) + pad
+    dist = -corners[:, 2]
+    pv = _ortho_reverse_z(x0, x1, y0, y1, dist.max() + pad, dist.min() - pad) @ view
+    return to_glm(pv)
+
+
 class FrameSequencer:
     """renderer.cpp:187-204: keeps last frame's view/proj and the post-incremented frame index.
 

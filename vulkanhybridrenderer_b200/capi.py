@@ -21,7 +21,7 @@ SYMBOLS = [
     "vhr_image_download", "vhr_storage_image_upload", "vhr_storage_image_download", "vhr_image_device_ptr",
     "vhr_storage_image_device_ptr", "vhr_bind_pass_images", "vhr_dispatch", "vhr_trace_rays",
     "vhr_blit_storage_to_transient", "vhr_blit_transient_to_storage", "vhr_blit_storage_to_storage", "vhr_set_option",
-    "vhr_get_option", "vhr_get_bvh_stats", "vhr_trace_explicit", "vhr_gbuffer_pass", "vhr_create_query_pool",
+    "vhr_get_option", "vhr_get_bvh_stats", "vhr_trace_explicit", "vhr_gbuffer_pass", "vhr_shadow_map_pass", "vhr_create_query_pool",
     "vhr_write_timestamp", "vhr_get_query_elapsed_ms", "vhr_debug_download_reflection_t",
     "vhr_image_upload_async", "vhr_image_download_async", "vhr_wait_download", "vhr_draw",
     "vhr_set_partition", "vhr_image_export_ipc", "vhr_storage_image_export_ipc", "vhr_image_attach_peer",
@@ -122,6 +122,7 @@ def lib():
         L.vhr_get_bvh_stats.argtypes = [vp, C.POINTER(BvhStats)]
         L.vhr_trace_explicit.argtypes = [vp, vp, u32, i32, vp, vp, vp]
         L.vhr_gbuffer_pass.argtypes = [vp, u32, u32]
+        L.vhr_shadow_map_pass.argtypes = [vp]
         L.vhr_draw.argtypes = [vp, C.c_char_p, C.POINTER(C.c_int32), u32, u32, u32, u32, u32]
         L.vhr_set_partition.argtypes = [vp, C.POINTER(Partition)]
         L.vhr_image_export_ipc.argtypes = [vp, C.c_char_p, vp]
@@ -388,6 +389,10 @@ class Context:
 
     def gbuffer_pass(self, width, height):
         _check(lib().vhr_gbuffer_pass(self._h, width, height))
+
+    def shadow_map_pass(self):
+        """Rasterises the scene into bound image 0 (the D32 Shadow Map) from directional_light.projview (vhr_shadow_map_pass)."""
+        _check(lib().vhr_shadow_map_pass(self._h))
 
     def blit_storage_to_transient(self, src, dst):
         _check(lib().vhr_blit_storage_to_transient(self._h, src, dst.encode()))

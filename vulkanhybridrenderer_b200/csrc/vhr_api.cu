@@ -217,6 +217,7 @@ void vhr_context_destroy(vhr_context *ctx) {
     for (auto &kv : ctx->transient) free_image(kv.second);
     for (auto &im : ctx->storage) if (im.used) free_image(im);
     free_bvh(ctx);
+    free_shadow_scratch(ctx);
     if (ctx->d_vertices) cudaFree(ctx->d_vertices);
     if (ctx->d_indices) cudaFree(ctx->d_indices);
     if (ctx->d_primitives) cudaFree(ctx->d_primitives);
@@ -678,6 +679,17 @@ int vhr_gbuffer_pass(vhr_context *ctx, uint32_t width, uint32_t height) {
     if (!ctx->pfd_set) return fail(VHR_ERR_STATE, "vhr_update_per_frame_ubo has not been called");
     VHR_CUDA_CHECK(cudaSetDevice(ctx->device));
     return launch_gbuffer(ctx, width, height);
+}
+
+int vhr_shadow_map_pass(vhr_context *ctx) {
+    if (ctx) ctx->epoch++;
+    NvtxRange nvtx_range("Shadow Map Pass");
+    if (!ctx) return fail(VHR_ERR_INVALID, "ctx is NULL");
+    VHR_NEED_DEVICE(ctx);
+    if (!ctx->pfd_set) return fail(VHR_ERR_STATE, "vhr_update_per_frame_ubo has not been called");
+    if (!ctx->d_primitives) return fail(VHR_ERR_STATE, "Shadow Map Pass: no geometry (vhr_update_geometry)");
+    VHR_CUDA_CHECK(cudaSetDevice(ctx->device));
+    return launch_shadow_map(ctx);
 }
 
 int vhr_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int any_hit, float *out_t, uint32_t *out_ids,

@@ -85,6 +85,15 @@ struct Partition {
     int no_exchange_step = 16;
 };
 // What a kernel needs to push its boundary rows into the neighbours' copies of the image it writes
+// Scratch of the shadow-map pass (shadow_map_kernels.cu): grows to the largest scene seen, freed with the context
+struct ShadowScratch {
+    void *counts = nullptr, *offsets = nullptr;      // uint64 per triangle + 1: tile counts and their exclusive scan
+    void *clip_list = nullptr;                       // uint32: [0] count, then the triangles that reach beyond the guard band
+    void *records = nullptr;                         // 48 B per triangle (written for large triangles only)
+    void *scan_tmp = nullptr;                        // CUB scan temporary storage
+    size_t counts_bytes = 0, offsets_bytes = 0, clip_list_bytes = 0, records_bytes = 0, scan_tmp_bytes = 0;
+    int sms = 0;
+};
 struct HaloPush {
     void *up = nullptr;       // same image on rank-1 (nullptr: no neighbour / no push)
     void *down = nullptr;     // same image on rank+1
@@ -125,6 +134,7 @@ struct vhr_context {
     size_t depth_tiles_count[2] = {0, 0};
     int raygen_blocks = 0;                         // resident grid of the persistent ray kernel (SMs x blocks/SM)
     vhr::Bvh bvh;
+    vhr::ShadowScratch shadow;
     vhr::Options opt;
     uint64_t launches = 0;
     uint32_t debug_label_depth = 0;                // open vhr_cmd_begin_debug_label ranges
@@ -174,6 +184,8 @@ int launch_gbuffer(vhr_context *ctx, uint32_t width, uint32_t height);
 int launch_raytraced(vhr_context *ctx, uint32_t width, uint32_t height);
 int launch_present(vhr_context *ctx);
 int launch_composition(vhr_context *ctx, int shadow_mode, int ao_mode, int reflection_mode);
+int launch_shadow_map(vhr_context *ctx);        // shadow_map_kernels.cu
+void free_shadow_scratch(vhr_context *ctx);
 int launch_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int any_hit, float *out_t, uint32_t *out_ids,
                           float *out_uv);
 // peer.cu: stream-ordered flag exchange with the other ranks (cuStreamWriteValue32 / cuStreamWaitValue32)

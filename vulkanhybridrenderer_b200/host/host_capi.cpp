@@ -205,6 +205,18 @@ int vhrh_set_gbuffer_producer(vhrh_renderer *r, int gbuffer_mode) {
     });
 }
 
+// shadow_map_mode 0 (the default): no producer, the pass records its draw calls and the harness may upload the Shadow Map itself;
+// 1: the CUDA depth rasteriser. The graph binds the pass's attachment ("Shadow Map", binding 0) before the hook runs.
+int vhrh_set_shadow_map_producer(vhrh_renderer *r, int shadow_map_mode) {
+    if (!r) return VHR_ERR_INVALID;
+    return guarded(r, [&] {
+        if (shadow_map_mode == 1)
+            r->render_graph->SetGraphicsPassHook("Shadow Map Pass", [](vhr_context *ctx) { VHR_CHECK(vhr_shadow_map_pass(ctx)); });
+        else
+            r->render_graph->SetGraphicsPassHook("Shadow Map Pass", nullptr);
+    });
+}
+
 // Renderer::Render (renderer.cpp:184-235): UBO update + RenderGraph::Execute; gather = GatherPerformanceStatistics
 int vhrh_render(vhrh_renderer *r, const void *per_frame_data, size_t size, int gather_statistics) {
     if (!r || !per_frame_data || size != sizeof(PerFrameData)) return VHR_ERR_INVALID;

@@ -201,7 +201,10 @@ void GraphicsExecutionContext::Draw(uint32_t vertex_count, uint32_t instance_cou
                        first_vertex, first_instance));
 }
 
-void RenderGraph::SetGraphicsPassHook(const std::string &pass_name, std::function<void(vhr_context *)> hook) { graphics_hooks[pass_name] = std::move(hook); }
+void RenderGraph::SetGraphicsPassHook(const std::string &pass_name, std::function<void(vhr_context *)> hook) {
+    if (hook) graphics_hooks[pass_name] = std::move(hook);
+    else graphics_hooks.erase(pass_name);
+}
 
 void RenderGraph::Execute(uint32_t resource_idx) {
     (void)resource_idx;   // the reference's 3 frames in flight collapse to stream order

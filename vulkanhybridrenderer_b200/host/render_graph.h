@@ -107,7 +107,8 @@ public:
     VkFormat GetImageFormat(const std::string &image_name) const;
 
     // What replaces the rasteriser for a graphics pass: called instead of recording draw calls (e.g. the CUDA G-buffer
-    // producer for "G-Buffer Pass"; nothing for "Composition Pass" when only the hot path is exercised).
+    // producer for "G-Buffer Pass"; nothing for "Composition Pass" when only the hot path is exercised). An empty `hook` removes
+    // the pass's hook: its draw calls are recorded again.
     void SetGraphicsPassHook(const std::string &pass_name, std::function<void(vhr_context *)> hook);
 
     std::vector<std::string> execution_order;

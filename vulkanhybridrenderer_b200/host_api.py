@@ -15,7 +15,7 @@ from . import types as T
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libvhr_host.so")
 SYMBOLS = ["vhrh_last_error", "vhrh_renderer_create", "vhrh_renderer_destroy", "vhrh_context", "vhrh_load_scene", "vhrh_set_modes",
-           "vhrh_set_gbuffer_producer", "vhrh_render", "vhrh_execution_order", "vhrh_pass_time_ms", "vhrh_svgf_push_constants",
+           "vhrh_set_gbuffer_producer", "vhrh_set_shadow_map_producer", "vhrh_render", "vhrh_execution_order", "vhrh_pass_time_ms", "vhrh_svgf_push_constants",
            "vhrh_parse_gltf", "vhrh_parsed_scene_destroy", "vhrh_parsed_scene_counts", "vhrh_parsed_scene_copy", "vhrh_parsed_scene_texture",
            "vhrh_load_gltf", "vhrh_decode_png", "vhrh_set_raytraced_path"]
 
@@ -44,6 +44,7 @@ def lib():
         L.vhrh_load_scene.argtypes = [vp, vp, u32, vp, u32, vp, u32, u32]
         L.vhrh_set_modes.argtypes = [vp, i32, i32, i32, i32, i32]
         L.vhrh_set_gbuffer_producer.argtypes = [vp, i32]
+        L.vhrh_set_shadow_map_producer.argtypes = [vp, i32]
         L.vhrh_render.argtypes = [vp, vp, C.c_size_t, i32]
         L.vhrh_execution_order.argtypes = [vp, C.c_char_p, C.c_size_t]
         L.vhrh_execution_order.restype = u32
@@ -118,6 +119,10 @@ class Renderer:
 
     def set_gbuffer_producer(self, cuda_primary_rays):
         _check(lib().vhrh_set_gbuffer_producer(self._r, 1 if cuda_primary_rays else 0))
+
+    def set_shadow_map_producer(self, cuda_rasteriser):
+        """True: the "Shadow Map Pass" node runs the CUDA depth rasteriser (vhr_shadow_map_pass); False: an external producer."""
+        _check(lib().vhrh_set_shadow_map_producer(self._r, 1 if cuda_rasteriser else 0))
 
     def render(self, pfd, gather_statistics=False):
         pfd = np.ascontiguousarray(pfd)

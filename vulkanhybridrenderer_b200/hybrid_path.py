@@ -177,6 +177,12 @@ class HybridRenderPath:
         pc["integrated_shadow_and_ao"] = pc["integrated_shadow_and_ao"][::-1].copy()
         self._stamp()
 
+    def shadow_map_pass(self):
+        """"Shadow Map Pass", hybrid_render_path.cpp:58-99: the Shadow Map as depth attachment 0, rasterised from the light."""
+        with self.ctx.debug_label("Shadow Map Pass"):
+            self.ctx.bind_pass_images([N_SHADOW_MAP])
+            self.ctx.shadow_map_pass()
+
     def composition_pass(self, shadow_mode=SHADOW_MODE_RAYTRACED, ao_mode=AO_MODE_RAYTRACED, reflection_mode=REFLECTION_MODE_OFF,
                          denoised=True, gset=0):
         """hybrid_render_path.cpp:333-379: nine sampled inputs by binding, RENDER_OUTPUT as colour attachment 0, Draw(3,1,0,0)."""
