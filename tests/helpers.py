@@ -45,6 +45,16 @@ def assert_parity(gpu, ref, what, max_abs=MAX_ABS_TOL, min_psnr=PSNR_MIN_DB, out
     return s
 
 
+def oracle_bilinear_setup(u, n):
+    """The oracle's bilinear_setup in numpy (float32 arrays): the filter coordinate t = fl(fl(u n) - 0.5) snapped to 1/256 as
+    floor(t 256 + 0.5) / 256; returns (texel floor, unwrapped, as int64; weight; t)."""
+    f32 = np.float32
+    uu = ((u * f32(n)).astype(f32) - f32(0.5)).astype(f32)
+    s = (np.floor(((uu * f32(256)).astype(f32) + f32(0.5)).astype(f32)) * f32(0.00390625)).astype(f32)
+    fl = np.floor(s)
+    return fl.astype(np.int64), (s - fl).astype(f32), uu
+
+
 @functools.lru_cache(maxsize=8)
 def scene_and_gbuffer(width, height, tris=20000, seed=3, moving=False):
     """Scene + oracle G-buffers of two consecutive frames (CPU primary rays; test scaffolding)."""
@@ -61,6 +71,72 @@ def scene_and_gbuffer(width, height, tris=20000, seed=3, moving=False):
         pfd = seq.next(cam)
         frames.append((pfd, osc.gbuffer(pfd, width, height)))
     return sc, osc, frames
+
+
+CAMERA_CASES = ("default", "jitter", "finite_far", "far_origin")
+
+
+@functools.lru_cache(maxsize=16)
+def camera_case(name, width, height):
+    """(scene, oracle scene, pfd, oracle G-buffer) of one camera of the screen-space parity tests:
+      default     the second frame of scene_and_gbuffer: infinite reverse-Z, whose inverse has only m00, m11, m23, m32 and m33 set;
+      jitter      a TAA-style sub-pixel offset in perspective[0, 2] and [1, 2]: the inverse is not sparse;
+      finite_far  reverse-Z with a far plane at 60: the inverse's m33 is not zero, so the sky (depth 0) unprojects with w != 0;
+      far_origin  scene and camera translated by ~10^3 (Primitive.transform and the camera pose): coordinates lose ten bits;
+      mirrored    perspective[0, 0] negated (a horizontally mirrored image);
+      narrow_fov  a 5e-5 rad vertical field of view: |camera_proj_inverse m00|, |m11| < 2^-14."""
+    if name == "default":
+        sc, osc, frames = scene_and_gbuffer(width, height)
+        return (sc, osc) + frames[1]
+    import checker as O
+    sc = scenes.sponza_like(20000, seed=3, width=width, height=height, n_clutter=40)
+    cam = sc.camera
+    if name == "jitter":
+        cam.perspective = cam.perspective.copy()
+        cam.perspective[0, 2], cam.perspective[1, 2] = 0.37 * 2.0 / width, -0.61 * 2.0 / height
+    elif name == "finite_far":
+        zn, zf = np.float32(cam.znear), np.float32(60.0)
+        cam.perspective = cam.perspective.copy()
+        cam.perspective[2, 2], cam.perspective[2, 3] = zn / (zf - zn), zn * zf / (zf - zn)
+    elif name == "far_origin":
+        off = np.array([1000.3, 250.7, -700.1])
+        sc.primitives = sc.primitives.copy()
+        sc.primitives["transform"][:, 3, :3] += off.astype(np.float32)
+        cam.set_pose(cam.position + off, cam.yaw, cam.pitch)
+    elif name == "mirrored":
+        cam.perspective = cam.perspective.copy()
+        cam.perspective[0, 0] = -cam.perspective[0, 0]
+    elif name == "narrow_fov":
+        cam.perspective = camera.infinite_reverse_depth_projection(5e-5, width / height, cam.znear)
+    else:
+        raise ValueError(name)
+    osc = O.OracleScene(sc)
+    seq = camera.FrameSequencer(width, height, sc.light)
+    seq.next(cam)
+    pfd = seq.next(cam)
+    return sc, osc, pfd, osc.gbuffer(pfd, width, height)
+
+
+def ssao_sample_angles(pfd, xs, ys):
+    """The 16 sample angles of SSAO pixels (xs, ys), [n, 16] float32: ssao.comp's seed_thread / random01 sequence (common.glsl:47-68;
+    the angle is fl(fl(r 2) PI) = fl(r (2 PI)), the distance draws the next number)."""
+    u32 = np.uint32
+    s = ((np.asarray(ys, np.uint64) * int(pfd["display_size"][1]) + np.asarray(xs, np.uint64)) * int(pfd["frame_index"])).astype(np.uint64)
+    s = (s & 0xFFFFFFFF).astype(u32)
+    with np.errstate(over="ignore"):
+        s = (s ^ u32(61)) ^ (s >> u32(16))
+        s = s * u32(9)
+        s = s ^ (s >> u32(4))
+        s = s * u32(0x27d4eb2d)
+        s = s ^ (s >> u32(15))
+        angles = []
+        for _ in range(16):
+            for k in range(2):
+                s = s ^ (s << u32(13)); s = s ^ (s >> u32(17)); s = s ^ (s << u32(5))
+                if k == 0:
+                    r = (u32(0x3f800000) | (s >> u32(9))).view(np.float32) - np.float32(1.0)
+                    angles.append((r * np.float32(2.0 * float(np.float32(np.pi)))).astype(np.float32))
+    return np.stack(angles, axis=-1)
 
 
 def noise_integrated(H, W, seed):

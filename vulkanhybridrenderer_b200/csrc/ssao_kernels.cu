@@ -429,10 +429,11 @@ int launch_ssao(vhr_context *ctx, uint32_t xg, uint32_t yg, float radius) {
     bool perspective = true;
     for (int i = 0; i < 16; ++i)
         if (i != 0 && i != 5 && i != 11 && i != 14 && i != 15 && ctx->pfd.camera_proj_inverse[i] != 0.0f) perspective = false;
-    // ... and its coefficients in the range occlusion_term<.., BOUNDED> relies on (any real camera: m00, m11 = tan(fov / 2) terms, m23 = -1)
+    // ... and its coefficients in the range occlusion_term<.., BOUNDED> relies on (any real camera: m00, m11 = tan(fov / 2) terms, m23 = -1);
+    // m00 and m11 positive, so that a zero dividend m00 x or m11 y is +0 (div_exact_flag_bounded's precondition: x = fl(2 u - 1) is never -0)
     {
         const float *m = ctx->pfd.camera_proj_inverse;
-        const float a0 = std::fabs(m[0]), a5 = std::fabs(m[5]), a14 = std::fabs(m[14]);
+        const float a0 = m[0], a5 = m[5], a14 = std::fabs(m[14]);
         if (!(a0 >= 6.1035156e-5f && a0 <= 256.0f && a5 >= 6.1035156e-5f && a5 <= 256.0f && a14 >= 3.6379788e-12f && a14 <= 2.7487791e11f)) perspective = false;
     }
     static const int variant = [] { const char *e = getenv("VHR_SSAO_VARIANT"); return e ? atoi(e) : 0; }();
