@@ -341,7 +341,18 @@ int vhr_debug_download_reflection_t(vhr_context *ctx, float *host, size_t bytes)
 
 /* G-buffer producer as a CUDA primary-ray pass (stand-in for the rasterised "G-Buffer Pass",
  * hybrid_render_path.cpp:13-56; encodings of gbuf.frag:33,43,46-58). Bound images: 0 albedo (BGRA8), 1 normals/ids,
- * 2 motion/metallic-roughness, 3 depth. */
+ * 2 motion/metallic-roughness, 3 depth.
+ * Without a partition it writes rows [VHR_OPT_ROW_BEGIN, VHR_OPT_ROW_END) of the bound images. Under a partition with world > 1
+ * every rank ends with the WHOLE G-buffer, bit-identical to the single-GPU pass: the rank traces the 8-row blocks its ray pass
+ * traces (ray_block_rows = 8: blocks b with b % world == rank) or its band (ray_block_rows = 0), and stores every texel, sky
+ * clears included, into its own four images and into the same texel of every other rank's (NVLink peer stores, 28 B per texel
+ * and peer). So every one of the four bound images needs a peer attached for every other rank (vhr_image_attach_peer[_pointer]);
+ * otherwise the call fails with VHR_ERR_STATE before anything is enqueued. After the kernel the call waits for all ranks (their
+ * rows have landed before any later pass reads them). Before the kernel it waits for all ranks too when the four images overlap
+ * those of the previous partitioned G-buffer pass since vhr_set_partition, or there was none: a peer may still be reading them.
+ * When the images differ (alternating G-buffer sets) that pass's trailing wait already ordered every rank's earlier work, so
+ * nothing is waited for; work that reads the other set after that pass is the caller's to order. As with every partitioned
+ * call, every rank must issue the same call sequence. */
 int vhr_gbuffer_pass(vhr_context *ctx, uint32_t width, uint32_t height);
 
 /* Shadow-map producer as a CUDA depth rasteriser (stand-in for the rasterised "Shadow Map Pass", hybrid_render_path.cpp:58-99,

@@ -123,6 +123,7 @@ extern "C" {
 
 int vhr_set_partition(vhr_context *ctx, const vhr_partition *p) {
     if (!ctx) return fail(VHR_ERR_INVALID, "ctx is NULL");
+    for (Image *&im : ctx->gbuffer_peer_written) im = nullptr;      // the next partitioned G-buffer pass starts with a leading sync
     if (!p) {      // back to single-GPU behaviour: the whole image is the dispatch range again
         ctx->part = Partition();
         ctx->opt.row_begin = 0;

@@ -14,6 +14,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "bvh.cuh"
@@ -1066,6 +1067,16 @@ struct GbufferParams {
     float *depth;
     SceneRefs scene;
 };
+// multi-GPU (a partition with world > 1): this rank traces its rows and stores every texel into its own four images AND the same
+// texel of every peer's, so each rank ends with the whole G-buffer. interleave = 1 (ray_block_rows = 8): the 8-row blocks b with
+// b % world == rank, exactly the blocks this rank's ray pass traces; interleave = 0: the rank's band [y_begin, y_end).
+struct GbufferPartParams : GbufferParams {
+    int world, rank, interleave;
+    uint32_t *albedo_of[VHR_MAX_RANKS];      // [rank] = this rank's own image
+    uint2 *normals_of[VHR_MAX_RANKS];
+    uint2 *motion_of[VHR_MAX_RANKS];
+    float *depth_of[VHR_MAX_RANKS];
+};
 
 __device__ __forceinline__ uint32_t unorm8(float f) {
     f = fminf(fmaxf(f, 0.0f), 1.0f);
@@ -1096,10 +1107,29 @@ __device__ __forceinline__ float3 cross_rn(float3 a, float3 b) {
     return make_float3(sub_rn(mul_rn(a.y, b.z), mul_rn(a.z, b.y)), sub_rn(mul_rn(a.z, b.x), mul_rn(a.x, b.z)), sub_rn(mul_rn(a.x, b.y), mul_rn(a.y, b.x)));
 }
 
-__global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ GbufferParams p, const __grid_constant__ PerFrameData pfd) {
+// partitioned instance: the texel goes to the same place in every rank's image (of[rank] is this rank's own)
+template <typename T>
+__device__ __forceinline__ void store_every_rank(T *const *of, int world, size_t i, T v) {
+#pragma unroll
+    for (int r = 0; r < VHR_MAX_RANKS; ++r)
+        if (r < world) of[r][i] = v;
+}
+
+// PART = false: the single-GPU pass over the rows [y_begin, y_end). PART = true (GbufferPartParams): the rows dealt to this rank,
+// every texel stored to every rank; the per-pixel arithmetic is the same.
+template <bool PART>
+__global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ std::conditional_t<PART, GbufferPartParams, GbufferParams> p,
+                                                      const __grid_constant__ PerFrameData pfd) {
     int x, y;
     tile_coords(x, y);
-    y += p.y_begin;
+    if constexpr (PART) {
+        if (p.interleave)      // blockIdx.y counts this rank's 8-row blocks, dealt as raygen_kernel deals them
+            y = (y - blockIdx.y * 8) + (blockIdx.y * p.world + p.rank) * 8;
+        else
+            y += p.y_begin;
+    } else {
+        y += p.y_begin;
+    }
     const bool in_range = x < p.W && y < p.y_end;       // trace() is warp-synchronous: no early return
     const size_t pix = in_range ? (size_t)y * p.W + x : 0;
     const float u = mul_rn(add_rn((float)x, 0.5f), pfd.display_size_inverse[0]);
@@ -1116,10 +1146,17 @@ __global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ Gb
     if (!in_range) return;
     if (!found) {
         // clear values of hybrid_render_path.cpp:16-19
-        if (p.albedo) p.albedo[pix] = 0u;
-        p.normals[pix] = make_uint2(0u, 0u);
-        p.motion[pix] = pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f));
-        p.depth[pix] = 0.0f;
+        if constexpr (PART) {
+            store_every_rank(p.albedo_of, p.world, pix, 0u);
+            store_every_rank(p.normals_of, p.world, pix, make_uint2(0u, 0u));
+            store_every_rank(p.motion_of, p.world, pix, pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f)));
+            store_every_rank(p.depth_of, p.world, pix, 0.0f);
+        } else {
+            if (p.albedo) p.albedo[pix] = 0u;
+            p.normals[pix] = make_uint2(0u, 0u);
+            p.motion[pix] = pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f));
+            p.depth[pix] = 0.0f;
+        }
         return;
     }
     const SceneRefs &s = p.scene;
@@ -1168,10 +1205,17 @@ __global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ Gb
     const float4 pclip = mul44_rn(pfd.camera_proj_prev_frame, mul44_rn(pfd.camera_view_prev_frame, pw));
     const float pu = add_rn(mul_rn(__fdiv_rn(pclip.x, pclip.w), 0.5f), 0.5f);
     const float pv = add_rn(mul_rn(__fdiv_rn(pclip.y, pclip.w), 0.5f), 0.5f);
-    if (p.albedo) p.albedo[pix] = unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24);
-    p.normals[pix] = pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g));
-    p.motion[pix] = pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness));
-    p.depth[pix] = __fdiv_rn(clip.z, clip.w);
+    if constexpr (PART) {
+        store_every_rank(p.albedo_of, p.world, pix, unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24));
+        store_every_rank(p.normals_of, p.world, pix, pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g)));
+        store_every_rank(p.motion_of, p.world, pix, pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness)));
+        store_every_rank(p.depth_of, p.world, pix, __fdiv_rn(clip.z, clip.w));
+    } else {
+        if (p.albedo) p.albedo[pix] = unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24);
+        p.normals[pix] = pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g));
+        p.motion[pix] = pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness));
+        p.depth[pix] = __fdiv_rn(clip.z, clip.w);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1332,6 +1376,14 @@ SceneRefs scene_refs(vhr_context *ctx) {
     return s;
 }
 
+std::string image_label(vhr_context *ctx, const Image *im) {
+    for (auto &kv : ctx->transient)
+        if (&kv.second == im) return "'" + kv.first + "'";
+    for (size_t s = 0; s < ctx->storage.size(); ++s)
+        if (&ctx->storage[s] == im) return "storage image " + std::to_string(s);
+    return "unknown image";
+}
+
 bool band(vhr_context *ctx, uint32_t height, int &y0, int &y1) {
     y0 = std::max(0, ctx->opt.row_begin);
     y1 = ctx->opt.row_end < 0 ? (int)height : std::min((int)height, ctx->opt.row_end);
@@ -1487,16 +1539,68 @@ int launch_gbuffer(vhr_context *ctx, uint32_t width, uint32_t height) {
         if (im->width != width || im->height != height) return fail(VHR_ERR_INVALID, "G-buffer pass: image size mismatch");
     for (Image *im : {albedo, normals, motion, depth})      // e.g. the normals image still shared with the SVGF pass's previous-frame copy
         if (int rc = make_writable(ctx, im, covers_image(ctx, im, width, height))) return rc;
-    GbufferParams p;
+    GbufferPartParams p;      // its GbufferParams part is all the single-GPU instance takes
     p.W = (int)width; p.H = (int)height;
     if (!band(ctx, height, p.y_begin, p.y_end)) return VHR_OK;
     p.albedo = (uint32_t *)albedo->ptr; p.normals = (uint2 *)normals->ptr; p.motion = (uint2 *)motion->ptr; p.depth = (float *)depth->ptr;
     p.scene = scene_refs(ctx);
-    dim3 block(128), grid((width + 15) / 16, (p.y_end - p.y_begin + 7) / 8);
-    gbuffer_kernel<<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
-    VHR_CUDA_CHECK(cudaGetLastError());
-    ctx->launches++;
-    return VHR_OK;
+    const Partition &pt = ctx->part;
+    if (!(pt.enabled && pt.world > 1)) {
+        dim3 block(128), grid((width + 15) / 16, (p.y_end - p.y_begin + 7) / 8);
+        gbuffer_kernel<false><<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
+        VHR_CUDA_CHECK(cudaGetLastError());
+        ctx->launches++;
+        return VHR_OK;
+    }
+    // Partitioned: this rank's rows go to every rank's images (include/vhr_b200.h). Every peer image must be attached before
+    // anything is enqueued, so that a failing call leaves no flag written and no stream waiting.
+    Image *const imgs[4] = {albedo, normals, motion, depth};
+    for (int i = 0; i < 4; ++i)
+        for (int r = 0; r < pt.world; ++r)
+            if (r != pt.rank && !imgs[i]->peer[r])
+                return fail(VHR_ERR_STATE, "G-buffer pass: binding %d (%s) has no image of rank %d attached (vhr_image_attach_peer)", i,
+                            image_label(ctx, imgs[i]).c_str(), r);
+    // Load the kernel before a flag wait is enqueued: with lazy module loading its first launch would otherwise wait for this stream, which
+    // then waits for the other ranks — a deadlock when they are contexts driven by this same thread and have not issued their signals yet.
+    static uint64_t loaded = 0;
+    if (!(loaded >> (ctx->device & 63) & 1ull)) {
+        cudaFuncAttributes attr;
+        VHR_CUDA_CHECK(cudaFuncGetAttributes(&attr, gbuffer_kernel<true>));
+        loaded |= 1ull << (ctx->device & 63);
+    }
+    p.world = pt.world; p.rank = pt.rank;
+    p.interleave = pt.ray_block_rows == 8;
+    for (int r = 0; r < pt.world; ++r) {
+        const bool own = r == pt.rank;
+        p.albedo_of[r] = (uint32_t *)(own ? albedo->ptr : albedo->peer[r]);
+        p.normals_of[r] = (uint2 *)(own ? normals->ptr : normals->peer[r]);
+        p.motion_of[r] = (uint2 *)(own ? motion->ptr : motion->peer[r]);
+        p.depth_of[r] = (float *)(own ? depth->ptr : depth->peer[r]);
+    }
+    // WAR on the peers' images: a peer may still be reading what the last partitioned G-buffer pass stored into these images. If that
+    // pass wrote other images (alternating G-buffer sets), its trailing sync already ordered every rank's earlier work before this
+    // one; otherwise (or with no such pass since the partition was installed) every rank first reaches this point.
+    bool reused = !ctx->gbuffer_peer_written[0];
+    for (Image *a : imgs)
+        for (Image *b : ctx->gbuffer_peer_written) reused |= a == b;
+    if (reused)
+        if (int rc = peer_sync_all(ctx)) return rc;
+    for (int i = 0; i < 4; ++i) ctx->gbuffer_peer_written[i] = imgs[i];
+    int rows;
+    if (p.interleave) {
+        p.y_begin = 0; p.y_end = (int)height;
+        const int n_blocks = ((int)height + 7) / 8;
+        rows = (n_blocks - pt.rank + pt.world - 1) / pt.world * 8;        // blocks b = rank, rank + world, ...
+    } else {
+        rows = p.y_end - p.y_begin;
+    }
+    if (rows > 0) {
+        dim3 block(128), grid((width + 15) / 16, (rows + 7) / 8);
+        gbuffer_kernel<true><<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
+        VHR_CUDA_CHECK(cudaGetLastError());
+        ctx->launches++;
+    }
+    return peer_sync_all(ctx);      // later passes read rows the other ranks stored; the ray pass may not follow (rasterised shadows)
 }
 
 int launch_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int any_hit, float *out_t, uint32_t *out_ids, float *out_uv) {

@@ -158,6 +158,7 @@ struct vhr_context {
     uint32_t *sync_flags = nullptr;                       // device: [0, MAX) ray-pass arrivals, [MAX, 2 MAX) halo arrivals, by source rank
     uint32_t *peer_flags[VHR_MAX_RANKS] = {};             // the other ranks' sync_flags (IPC mapped)
     uint32_t seq_ray = 0, seq_halo = 0;
+    vhr::Image *gbuffer_peer_written[4] = {};             // the images the last partitioned G-buffer pass stored to every rank (none: cleared by vhr_set_partition)
     std::vector<void *> ipc_opened;                       // everything cudaIpcOpenMemHandle returned (closed with the context)
 };
 

@@ -177,6 +177,16 @@ class HybridRenderPath:
         pc["integrated_shadow_and_ao"] = pc["integrated_shadow_and_ao"][::-1].copy()
         self._stamp()
 
+    def gbuffer_pass(self, gset=0):
+        """"G-Buffer Pass", hybrid_render_path.cpp:13-56: G-buffer set `gset` (0 albedo, 1 normals/ids, 2 motion/metallic-roughness,
+        3 depth) produced by primary rays for the per-frame constants last uploaded. Under a fused partition whose G-buffer sets are
+        exchanged (multi_gpu.setup_fused_partition(..., exchange_gbuffer=True)) every rank traces its own rows and ends with the whole
+        G-buffer."""
+        g = self.gsets[gset]
+        with self.ctx.debug_label("G-Buffer Pass"):
+            self.ctx.bind_pass_images([g[N_ALBEDO], g[N_NORMALS], g[N_MOTION], g[N_DEPTH]])
+            self.ctx.gbuffer_pass(self.W, self.H)
+
     def shadow_map_pass(self):
         """"Shadow Map Pass", hybrid_render_path.cpp:58-99: the Shadow Map as depth attachment 0, rasterised from the light."""
         with self.ctx.debug_label("Shadow Map Pass"):

@@ -167,17 +167,25 @@ def _has_image(ctx, name):
         return False
 
 
-def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray_block_rows=8):
+def _gbuffer_names(path):
+    from . import hybrid_path as HP
+    return [g[k] for g in path.gsets for k in (HP.N_ALBEDO, HP.N_NORMALS, HP.N_MOTION, HP.N_DEPTH)]
+
+
+def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False):
     """Exports this rank's exchanged images, attaches everybody else's, installs the row partition on `ctx`.
 
     Exchanged images: the ray pass outputs (every rank stores into every owner's), the two integrated ping-pong images and
     the moments image with its twin (boundary rows pushed to the two neighbours). After this the plain single-GPU call
-    sequence (`HybridRenderPath.frame`) runs the partitioned frame."""
+    sequence (`HybridRenderPath.frame`) runs the partitioned frame.
+    exchange_gbuffer: also the four images of every G-buffer set, attached for all ranks, so that `HybridRenderPath.gbuffer_pass`
+    runs partitioned (every rank traces its rows and stores them into every rank's G-buffer): the frame is driven from a camera."""
     import torch.distributed as dist
     pc = path.pc
     mine = {"sync": ctx.sync_export_ipc(), "rt": [], "integ": [], "moments": None}
     for rt_name, refl_name in path.rt_sets:
         mine["rt"].append((ctx.image_export_ipc(rt_name), ctx.image_export_ipc(refl_name)))
+    mine["gbuffer"] = [ctx.image_export_ipc(n) for n in _gbuffer_names(path)] if exchange_gbuffer else []
     for slot in pc["integrated_shadow_and_ao"]:
         mine["integ"].append((int(slot), ctx.storage_image_export_ipc(int(slot))[0]))
     mslot = int(pc["shadow_and_ao_moments_history"])
@@ -194,6 +202,8 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
         for (rt_name, refl_name), (h_rt, h_refl) in zip(path.rt_sets, other["rt"]):
             ctx.image_attach_peer(rt_name, r, h_rt)
             ctx.image_attach_peer(refl_name, r, h_refl)
+        for name, h in zip(_gbuffer_names(path), other["gbuffer"]):
+            ctx.image_attach_peer(name, r, h)
         if abs(r - rank) == 1:                       # halos only ever go to the two neighbours
             for (slot, _), (_, h) in zip(mine["integ"], other["integ"]):
                 ctx.storage_image_attach_peer(slot, r, h)
@@ -206,10 +216,11 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
     return bands
 
 
-def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8):
+def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False):
     """The same partition for ranks that live in ONE process (one context per rank, all driven by this thread): peers are
     attached by plain device pointer. With all contexts on one GPU this exercises the whole fused path — interleaved ray
-    blocks, halo pushes, flag-word ordering between the streams — on a single-GPU box (tests/test_partition_gpu.py)."""
+    blocks, halo pushes, flag-word ordering between the streams — on a single-GPU box (tests/test_partition_gpu.py).
+    exchange_gbuffer: as for setup_fused_partition."""
     from . import capi
     L = capi.lib()
     world = len(ctxs)
@@ -222,6 +233,9 @@ def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8
             for (rt_name, refl_name), (ort, orefl) in zip(path.rt_sets, opath.rt_sets):
                 capi._check(L.vhr_image_attach_peer_pointer(ctx._h, rt_name.encode(), q, octx.image_info(ort)[0]))
                 capi._check(L.vhr_image_attach_peer_pointer(ctx._h, refl_name.encode(), q, octx.image_info(orefl)[0]))
+            if exchange_gbuffer:
+                for name, oname in zip(_gbuffer_names(path), _gbuffer_names(opath)):
+                    capi._check(L.vhr_image_attach_peer_pointer(ctx._h, name.encode(), q, octx.image_info(oname)[0]))
             if abs(q - r) == 1:
                 for slot, oslot in zip(path.pc["integrated_shadow_and_ao"], opath.pc["integrated_shadow_and_ao"]):
                     capi._check(L.vhr_storage_image_attach_peer_pointer(ctx._h, int(slot), q, octx.storage_image_info(int(oslot))[0], None))
