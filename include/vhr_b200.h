@@ -363,8 +363,19 @@ int vhr_gbuffer_pass(vhr_context *ctx, uint32_t width, uint32_t height);
  * the exact arithmetic; the result does not depend on the order of the triangles. projview must be finite with a last row
  * of (0, 0, 0, 1) (an orthographic light, as the scene loader builds) or all zero (a scene without a light: the map is only
  * cleared); anything else is VHR_ERR_INVALID. VHR_ERR_STATE without geometry or per-frame constants; VHR_ERR_CUDA on a
- * VHR_DEVICE_NONE context. VHR_OPT_ROW_BEGIN / END do not apply (the map is not display-sized), and under a partition every
- * rank renders the whole map (replicated input, like the acceleration structure). Runs on the selected queue. */
+ * VHR_DEVICE_NONE context. VHR_OPT_ROW_BEGIN / END do not apply (the map is not display-sized). Runs on the selected queue.
+ * Without a partition, with world == 1, or when the bound map has no peer attached for any other rank, every rank renders
+ * the whole map (replicated input, like the acceleration structure). Under a partition with world > 1 and the map attached for
+ * every other rank (vhr_image_attach_peer[_pointer]) the pass runs partitioned and every rank ends with the WHOLE map,
+ * bit-identical to the single-GPU pass: the map's rows are dealt in blocks of 8 (block b to rank b % world; a rank of a tiny
+ * map may own none), each rank projects every triangle but rasterises only the samples of its own rows, clears and fills
+ * those rows of its map and stores them into the same rows of every other rank's map (NVLink peer stores, 4 B per texel and
+ * peer). The call waits for all ranks before it (a peer may still be reading its map) and after the push (every rank's rows
+ * have landed before any later pass reads the map). The cleared-map cases (zero projview, no triangles) run the same way.
+ * With the map attached for some other ranks but not all, the call fails with VHR_ERR_STATE naming the missing rank; that
+ * check and the ones above run before any flag word is written or waited on. Which path runs is decided on each rank alone, so
+ * every rank must attach the map the same way: a rank with every peer attached waits for flag words that a rank with none
+ * attached never writes. As with every partitioned call, every rank must issue the same call sequence. */
 int vhr_shadow_map_pass(vhr_context *ctx);
 
 #ifdef __cplusplus

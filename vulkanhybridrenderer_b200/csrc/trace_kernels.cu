@@ -1376,14 +1376,6 @@ SceneRefs scene_refs(vhr_context *ctx) {
     return s;
 }
 
-std::string image_label(vhr_context *ctx, const Image *im) {
-    for (auto &kv : ctx->transient)
-        if (&kv.second == im) return "'" + kv.first + "'";
-    for (size_t s = 0; s < ctx->storage.size(); ++s)
-        if (&ctx->storage[s] == im) return "storage image " + std::to_string(s);
-    return "unknown image";
-}
-
 bool band(vhr_context *ctx, uint32_t height, int &y0, int &y1) {
     y0 = std::max(0, ctx->opt.row_begin);
     y1 = ctx->opt.row_end < 0 ? (int)height : std::min((int)height, ctx->opt.row_end);

@@ -103,6 +103,14 @@ static int copy_out(vhr_context *ctx, Image *im, void *host, size_t bytes, const
 }
 }  // namespace vhr (anonymous part)
 
+std::string vhr::image_label(vhr_context *ctx, const Image *im) {
+    for (auto &kv : ctx->transient)
+        if (&kv.second == im) return "'" + kv.first + "'";
+    for (size_t s = 0; s < ctx->storage.size(); ++s)
+        if (&ctx->storage[s] == im) return "storage image " + std::to_string(s);
+    return "unknown image";
+}
+
 int vhr::make_writable(vhr_context *ctx, Image *im, bool whole) {
     if (im && im->direct_read_pending) {      // a row read-back straight from the image (vhr_image_download_rows_async) is still in flight
         VHR_CUDA_CHECK(cudaStreamWaitEvent(ctx->stream, im->direct_read_done, 0));

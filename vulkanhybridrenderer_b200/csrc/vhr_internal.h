@@ -93,6 +93,7 @@ struct ShadowScratch {
     void *scan_tmp = nullptr;                        // CUB scan temporary storage
     size_t counts_bytes = 0, offsets_bytes = 0, clip_list_bytes = 0, records_bytes = 0, scan_tmp_bytes = 0;
     int sms = 0;
+    std::vector<void *> retired;                     // buffers a partitioned pass outgrew: freed without a device synchronisation later
 };
 struct HaloPush {
     void *up = nullptr;       // same image on rank-1 (nullptr: no neighbour / no push)
@@ -197,6 +198,8 @@ void peer_close_all(vhr_context *ctx);
 // Call before enqueueing work that writes `im`: an image that shares its buffer with a blit partner gets the spare allocation
 // (its old content is copied over first unless the write covers the `whole` image). No-op for images that share nothing.
 int make_writable(vhr_context *ctx, Image *im, bool whole);
+// "'name'" of a transient image, "storage image <slot>" of a storage image (error messages)
+std::string image_label(vhr_context *ctx, const Image *im);
 // does a pass dispatched over xg x yg groups of 8 x 8 (or a w x h launch) overwrite every texel of `im`?
 inline bool covers_image(const vhr_context *ctx, const Image *im, uint64_t w, uint64_t h) {
     return !ctx->part.enabled && ctx->opt.row_begin <= 0 && (ctx->opt.row_end < 0 || ctx->opt.row_end >= (int)im->height) && w >= im->width && h >= im->height;

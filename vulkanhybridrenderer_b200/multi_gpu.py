@@ -172,20 +172,25 @@ def _gbuffer_names(path):
     return [g[k] for g in path.gsets for k in (HP.N_ALBEDO, HP.N_NORMALS, HP.N_MOTION, HP.N_DEPTH)]
 
 
-def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False):
+def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False,
+                          exchange_shadow_map=False):
     """Exports this rank's exchanged images, attaches everybody else's, installs the row partition on `ctx`.
 
     Exchanged images: the ray pass outputs (every rank stores into every owner's), the two integrated ping-pong images and
     the moments image with its twin (boundary rows pushed to the two neighbours). After this the plain single-GPU call
     sequence (`HybridRenderPath.frame`) runs the partitioned frame.
     exchange_gbuffer: also the four images of every G-buffer set, attached for all ranks, so that `HybridRenderPath.gbuffer_pass`
-    runs partitioned (every rank traces its rows and stores them into every rank's G-buffer): the frame is driven from a camera."""
+    runs partitioned (every rank traces its rows and stores them into every rank's G-buffer): the frame is driven from a camera.
+    exchange_shadow_map: also the "Shadow Map", attached for all ranks, so that `HybridRenderPath.shadow_map_pass` runs partitioned
+    (every rank rasterises its 8-row blocks of the map and stores them into every rank's map)."""
     import torch.distributed as dist
+    from . import hybrid_path as HP
     pc = path.pc
     mine = {"sync": ctx.sync_export_ipc(), "rt": [], "integ": [], "moments": None}
     for rt_name, refl_name in path.rt_sets:
         mine["rt"].append((ctx.image_export_ipc(rt_name), ctx.image_export_ipc(refl_name)))
     mine["gbuffer"] = [ctx.image_export_ipc(n) for n in _gbuffer_names(path)] if exchange_gbuffer else []
+    mine["shadow_map"] = ctx.image_export_ipc(HP.N_SHADOW_MAP) if exchange_shadow_map else None
     for slot in pc["integrated_shadow_and_ao"]:
         mine["integ"].append((int(slot), ctx.storage_image_export_ipc(int(slot))[0]))
     mslot = int(pc["shadow_and_ao_moments_history"])
@@ -204,6 +209,8 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
             ctx.image_attach_peer(refl_name, r, h_refl)
         for name, h in zip(_gbuffer_names(path), other["gbuffer"]):
             ctx.image_attach_peer(name, r, h)
+        if other["shadow_map"] is not None:
+            ctx.image_attach_peer(HP.N_SHADOW_MAP, r, other["shadow_map"])
         if abs(r - rank) == 1:                       # halos only ever go to the two neighbours
             for (slot, _), (_, h) in zip(mine["integ"], other["integ"]):
                 ctx.storage_image_attach_peer(slot, r, h)
@@ -216,12 +223,12 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
     return bands
 
 
-def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False):
+def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False, exchange_shadow_map=False):
     """The same partition for ranks that live in ONE process (one context per rank, all driven by this thread): peers are
     attached by plain device pointer. With all contexts on one GPU this exercises the whole fused path — interleaved ray
     blocks, halo pushes, flag-word ordering between the streams — on a single-GPU box (tests/test_partition_gpu.py).
-    exchange_gbuffer: as for setup_fused_partition."""
-    from . import capi
+    exchange_gbuffer, exchange_shadow_map: as for setup_fused_partition."""
+    from . import capi, hybrid_path as HP
     L = capi.lib()
     world = len(ctxs)
     H = paths[0].H
@@ -236,6 +243,8 @@ def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8
             if exchange_gbuffer:
                 for name, oname in zip(_gbuffer_names(path), _gbuffer_names(opath)):
                     capi._check(L.vhr_image_attach_peer_pointer(ctx._h, name.encode(), q, octx.image_info(oname)[0]))
+            if exchange_shadow_map:
+                capi._check(L.vhr_image_attach_peer_pointer(ctx._h, HP.N_SHADOW_MAP.encode(), q, octx.image_info(HP.N_SHADOW_MAP)[0]))
             if abs(q - r) == 1:
                 for slot, oslot in zip(path.pc["integrated_shadow_and_ao"], opath.pc["integrated_shadow_and_ao"]):
                     capi._check(L.vhr_storage_image_attach_peer_pointer(ctx._h, int(slot), q, octx.storage_image_info(int(oslot))[0], None))
