@@ -192,7 +192,19 @@ int vhr_trace_rays(vhr_context *ctx, const char *pipeline_name, uint32_t width, 
  * reference's swapchain: sRGB-encoded on store), B8G8R8A8_UNORM, or R16G16B16A16_SFLOAT (linear HDR radiance, for
  * parity measurements). "raytraced_render_path/composition.frag" (raytraced_render_path.cpp:49-76; no constants) copies
  * bound image 0 (RaytracedOutput) to the attachment at index 1, sRGB-encoding when it is B8G8R8A8_SRGB.
- * Any other shader or draw shape fails with VHR_ERR_INVALID (there is no rasteriser). */
+ * Any other shader or draw shape fails with VHR_ERR_INVALID (there is no rasteriser).
+ * Both draws write rows [VHR_OPT_ROW_BEGIN, VHR_OPT_ROW_END) of the attachment, under a partition the rank's band. Gathered output:
+ * under a partition with world > 1 and VHR_OPT_OUTPUT_RANK = p >= 0, rank p's attachment holds the WHOLE frame after the draw,
+ * bit-identical to the single-GPU draw: every other rank stores each texel of its band a second time, with the same bits, into the
+ * same texel of rank p's attachment (NVLink peer stores, 4 or 8 B per texel), so the attachment needs rank p's image attached on
+ * every rank but p (vhr_image_attach_peer[_pointer]). Every other rank's attachment holds its band as without the option; its rows
+ * outside the band are untouched. The call enqueues: a wait for a row read-back of the attachment still in flight, a wait for all
+ * ranks (rank p may still be reading its previous frame's output), the one kernel, and a wait for all ranks (every band has landed
+ * before anything on rank p reads the attachment). p >= world fails with VHR_ERR_INVALID on every rank; a rank other than p without
+ * rank p's attachment fails with VHR_ERR_STATE naming the image and the rank. Both checks run before any flag word is written or
+ * waited on. Which path runs is decided on each rank alone, so every rank must set the same output rank and attach p's output the
+ * same way: a rank that fails, or that does not gather, leaves the others waiting for flag words it never writes. As with every
+ * partitioned call, every rank must issue the same call sequence. */
 int vhr_draw(vhr_context *ctx, const char *fragment_shader, const int32_t *specialization_constants, uint32_t n_constants,
              uint32_t vertex_count, uint32_t instance_count, uint32_t first_vertex, uint32_t first_instance);
 
@@ -302,12 +314,16 @@ typedef enum vhr_option {
                                       Same images in every variant; all measured equal to or slower than 0 on B200, kept for study (DESIGN.md) */
     VHR_OPT_RAYTRACED_ALPHA_TEST = 11,/* the fully ray-traced path's use_anyhit_shader (raytraced_render_path.h:14): 1 selects the pipeline
                                       raygen_test_alpha.rgen + closesthit_test_alpha.rchit + shadow_anyhit.rahit */
-    VHR_OPT_BLIT_ALIAS = 12        /* 1: the three vhr_blit_* calls stop copying. After a blit source and destination show one buffer;
+    VHR_OPT_BLIT_ALIAS = 12,       /* 1: the three vhr_blit_* calls stop copying. After a blit source and destination show one buffer;
                                       whichever of the two is written next (a kernel output, an upload, another blit) takes the
                                       allocation the destination gave up, so every image always holds what the copy would have left
                                       (copy-on-write). Removes the three copies of the SVGF pass (hybrid_render_path.cpp:309-325: 48 B/px).
                                       Device pointers obtained through vhr_*_device_ptr are invalidated by blits and writes while it is on;
                                       ignored (real copies) while a multi-GPU partition is installed. Default 0 */
+    VHR_OPT_OUTPUT_RANK = 13       /* -1 (default): off. p in [0, VHR_MAX_RANKS): under a partition with world > 1 the composition draws
+                                      (vhr_draw) gather the whole frame into rank p's render output; see vhr_draw. Every rank must set
+                                      the same value and attach p's render output the same way. Ignored without a partition or with
+                                      world == 1. Other values: VHR_ERR_INVALID */
 } vhr_option;
 int vhr_set_option(vhr_context *ctx, int option, int64_t value);
 int64_t vhr_get_option(vhr_context *ctx, int option);

@@ -46,6 +46,7 @@ OPT_AO_SPP, OPT_TRACE_SHADOWS, OPT_TRACE_AO, OPT_TRACE_REFLECTIONS = 1, 2, 3, 4
 OPT_ROW_BEGIN, OPT_ROW_END, OPT_SVGF_FUSED, OPT_ATROUS_VARIANT, OPT_DEBUG_REFLECTION_T, OPT_RAYGEN_VARIANT = 5, 6, 7, 8, 9, 10
 OPT_RAYTRACED_ALPHA_TEST = 11
 OPT_BLIT_ALIAS = 12
+OPT_OUTPUT_RANK = 13
 
 
 class SamplerInfo(C.Structure):

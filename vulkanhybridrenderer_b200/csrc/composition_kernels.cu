@@ -11,7 +11,12 @@
 // Output formats: B8G8R8A8_SRGB (the reference's swapchain, vulkan_context.cpp:331: linear -> sRGB encode on store),
 // B8G8R8A8_UNORM (no encode) or R16G16B16A16_SFLOAT (linear HDR, what the parity tests compare). NaN stores as 0, like
 // the float -> UNORM conversion of the reference's attachment write (sky pixels: the unprojection divides by w = 0).
+//
+// Gathered output (VHR_OPT_OUTPUT_RANK under a partition): the <GATHER = true> instances store every texel of the rank's band a second
+// time, with the same bits, into the output rank's RENDER_OUTPUT over NVLink, so that rank ends with the whole frame. The <false>
+// instances are the single-GPU kernels; the output rank itself runs them too.
 #include <algorithm>
+#include <type_traits>
 
 #include "vhr_internal.h"
 
@@ -34,6 +39,9 @@ struct CompositionParams {
     const void *rt;                // binding 7
     const uint2 *refl;             // binding 8
     void *out;                     // attachment 0
+};
+struct CompositionGatherParams : CompositionParams {
+    void *out_gather;              // the output rank's render output
 };
 
 // Divisions, square roots and the sRGB power run on the MUFU unit (rcp / rsq / lg2 / ex2, <= 2 ulp) instead of the IEEE
@@ -69,8 +77,9 @@ __device__ __forceinline__ float sample_shadow_map(const CompositionParams &p, f
 // The three modes are template parameters, the CUDA counterpart of the reference's specialisation constants
 // (composition.frag:6-8, hybrid_render_path.cpp:361-369): each of the 27 pipelines carries only the loads and the
 // arithmetic of its own mode.
-template <int SHADOW_MODE, int AO_MODE, int REFLECTION_MODE>
-__global__ void __launch_bounds__(256) composition_kernel(const __grid_constant__ CompositionParams p, const __grid_constant__ PerFrameData pfd) {
+template <int SHADOW_MODE, int AO_MODE, int REFLECTION_MODE, bool GATHER>
+__global__ void __launch_bounds__(256) composition_kernel(const __grid_constant__ std::conditional_t<GATHER, CompositionGatherParams, CompositionParams> p,
+                                                          const __grid_constant__ PerFrameData pfd) {
     const int x = blockIdx.x * 64 + threadIdx.x;        // blockDim = (64, 4): 512-byte rows of 8-byte texels per warp pair
     const int y = p.y_begin + blockIdx.y * 4 + threadIdx.y;
     if (x >= p.W || y >= p.y_end) return;
@@ -174,11 +183,15 @@ __global__ void __launch_bounds__(256) composition_kernel(const __grid_constant_
         lighting.x = (lighting.x == lighting.x) ? lighting.x : 0.0f;
         lighting.y = (lighting.y == lighting.y) ? lighting.y : 0.0f;
         lighting.z = (lighting.z == lighting.z) ? lighting.z : 0.0f;
-        reinterpret_cast<uint2 *>(p.out)[pix] = pack_rgba16f(make_float4(lighting.x, lighting.y, lighting.z, 1.0f));
+        const uint2 c = pack_rgba16f(make_float4(lighting.x, lighting.y, lighting.z, 1.0f));
+        reinterpret_cast<uint2 *>(p.out)[pix] = c;
+        if constexpr (GATHER) reinterpret_cast<uint2 *>(p.out_gather)[pix] = c;
     } else {
         float r = lighting.x, g = lighting.y, b = lighting.z;
         if (p.out_format == VHR_FORMAT_B8G8R8A8_SRGB) { r = srgb_encode(r); g = srgb_encode(g); b = srgb_encode(b); }
-        reinterpret_cast<uint32_t *>(p.out)[pix] = unorm8_rn(b) | (unorm8_rn(g) << 8) | (unorm8_rn(r) << 16) | 0xff000000u;
+        const uint32_t c = unorm8_rn(b) | (unorm8_rn(g) << 8) | (unorm8_rn(r) << 16) | 0xff000000u;
+        reinterpret_cast<uint32_t *>(p.out)[pix] = c;
+        if constexpr (GATHER) reinterpret_cast<uint32_t *>(p.out_gather)[pix] = c;
     }
 }
 
@@ -189,18 +202,62 @@ struct PresentParams {
     const uint32_t *in;      // binding 0: RaytracedOutput, B8G8R8A8_UNORM
     void *out;
 };
-__global__ void __launch_bounds__(256) present_kernel(const __grid_constant__ PresentParams p) {
+struct PresentGatherParams : PresentParams {
+    void *out_gather;        // the output rank's render output
+};
+template <bool GATHER>
+__global__ void __launch_bounds__(256) present_kernel(const __grid_constant__ std::conditional_t<GATHER, PresentGatherParams, PresentParams> p) {
     const int x = blockIdx.x * 64 + threadIdx.x, y = p.y_begin + blockIdx.y * 4 + threadIdx.y;
     if (x >= p.W || y >= p.y_end) return;
     const size_t pix = (size_t)y * p.W + x;
     const uint32_t c = __ldg(&p.in[pix]);
-    if (p.out_format == VHR_FORMAT_B8G8R8A8_UNORM) { reinterpret_cast<uint32_t *>(p.out)[pix] = c; return; }
-    const float b = fdiv((float)(c & 0xffu), 255.0f), g = fdiv((float)((c >> 8) & 0xffu), 255.0f), r = fdiv((float)((c >> 16) & 0xffu), 255.0f);
-    if (p.out_format == VHR_FORMAT_R16G16B16A16_SFLOAT) {
-        reinterpret_cast<uint2 *>(p.out)[pix] = pack_rgba16f(make_float4(r, g, b, fdiv((float)(c >> 24), 255.0f)));
+    if (p.out_format == VHR_FORMAT_B8G8R8A8_UNORM) {
+        reinterpret_cast<uint32_t *>(p.out)[pix] = c;
+        if constexpr (GATHER) reinterpret_cast<uint32_t *>(p.out_gather)[pix] = c;
         return;
     }
-    reinterpret_cast<uint32_t *>(p.out)[pix] = unorm8_rn(srgb_encode(b)) | (unorm8_rn(srgb_encode(g)) << 8) | (unorm8_rn(srgb_encode(r)) << 16) | (c & 0xff000000u);
+    const float b = fdiv((float)(c & 0xffu), 255.0f), g = fdiv((float)((c >> 8) & 0xffu), 255.0f), r = fdiv((float)((c >> 16) & 0xffu), 255.0f);
+    if (p.out_format == VHR_FORMAT_R16G16B16A16_SFLOAT) {
+        const uint2 h = pack_rgba16f(make_float4(r, g, b, fdiv((float)(c >> 24), 255.0f)));
+        reinterpret_cast<uint2 *>(p.out)[pix] = h;
+        if constexpr (GATHER) reinterpret_cast<uint2 *>(p.out_gather)[pix] = h;
+        return;
+    }
+    const uint32_t e = unorm8_rn(srgb_encode(b)) | (unorm8_rn(srgb_encode(g)) << 8) | (unorm8_rn(srgb_encode(r)) << 16) | (c & 0xff000000u);
+    reinterpret_cast<uint32_t *>(p.out)[pix] = e;
+    if constexpr (GATHER) reinterpret_cast<uint32_t *>(p.out_gather)[pix] = e;
+}
+
+// VHR_OPT_OUTPUT_RANK (include/vhr_b200.h): `gather` = this draw gathers the frame on the output rank; `peer_out` = where this rank's
+// texels go a second time (nullptr on the output rank itself, which only receives). Every failure comes before anything is enqueued,
+// so a rank that fails leaves no flag written and no stream waiting.
+static int gather_target(vhr_context *ctx, Image *out, const char *what, bool &gather, void *&peer_out) {
+    const Partition &pt = ctx->part;
+    const int p = ctx->opt.output_rank;
+    gather = pt.enabled && pt.world > 1 && p >= 0;
+    peer_out = nullptr;
+    if (!gather) return VHR_OK;
+    if (p >= pt.world) return fail(VHR_ERR_INVALID, "%s: VHR_OPT_OUTPUT_RANK %d is not a rank of the partition (world %d)", what, p, pt.world);
+    if (p == pt.rank) return VHR_OK;
+    peer_out = out->peer[p];
+    if (!peer_out)
+        return fail(VHR_ERR_STATE, "%s: the render output (%s) has no image of rank %d attached (vhr_image_attach_peer)", what,
+                    image_label(ctx, out).c_str(), p);
+    return VHR_OK;
+}
+
+// Load both instances a gathering draw may launch before its leading flag wait is enqueued: with lazy module loading a first launch
+// would otherwise wait for this stream, which then waits for the other ranks — a deadlock when they are contexts driven by this same
+// thread and have not issued their signals yet. `slot` tells the 27 mode combinations and present_kernel (27) apart.
+template <typename K0, typename K1>
+static int load_pair(vhr_context *ctx, int slot, K0 k0, K1 k1) {
+    static uint64_t loaded[28] = {};
+    if (loaded[slot] >> (ctx->device & 63) & 1ull) return VHR_OK;
+    cudaFuncAttributes attr;
+    VHR_CUDA_CHECK(cudaFuncGetAttributes(&attr, k0));
+    VHR_CUDA_CHECK(cudaFuncGetAttributes(&attr, k1));
+    loaded[slot] |= 1ull << (ctx->device & 63);
+    return VHR_OK;
 }
 
 int launch_present(vhr_context *ctx) {
@@ -211,18 +268,29 @@ int launch_present(vhr_context *ctx) {
     if (out->format != VHR_FORMAT_B8G8R8A8_SRGB && out->format != VHR_FORMAT_B8G8R8A8_UNORM && out->format != VHR_FORMAT_R16G16B16A16_SFLOAT)
         return fail(VHR_ERR_INVALID, "raytraced composition: render output format %d", out->format);
     if (in->width != out->width || in->height != out->height) return fail(VHR_ERR_INVALID, "raytraced composition: image sizes differ");
+    bool gather;
+    void *peer_out;
+    if (int rc = gather_target(ctx, out, "raytraced composition", gather, peer_out)) return rc;
+    if (gather)
+        if (int rc = load_pair(ctx, 27, present_kernel<false>, present_kernel<true>)) return rc;
     if (int rc = make_writable(ctx, out, covers_image(ctx, out, out->width, out->height))) return rc;
-    PresentParams p;
+    PresentGatherParams p;      // its PresentParams part is all the <false> instance takes
     p.W = (int)out->width; p.H = (int)out->height;
     p.y_begin = std::max(0, ctx->opt.row_begin);
     p.y_end = ctx->opt.row_end < 0 ? p.H : std::min(p.H, ctx->opt.row_end);
-    if (p.y_end <= p.y_begin) return VHR_OK;
-    p.out_format = out->format; p.in = (const uint32_t *)in->ptr; p.out = out->ptr;
-    dim3 block(64, 4), grid((p.W + 63) / 64, (p.y_end - p.y_begin + 3) / 4);
-    present_kernel<<<grid, block, 0, ctx->stream>>>(p);
-    VHR_CUDA_CHECK(cudaGetLastError());
-    ctx->launches++;
-    return VHR_OK;
+    if (p.y_end <= p.y_begin && !gather) return VHR_OK;
+    p.out_format = out->format; p.in = (const uint32_t *)in->ptr; p.out = out->ptr; p.out_gather = peer_out;
+    // gathering: the output rank may still read the previous frame's output (nothing else orders that on this path)
+    if (gather)
+        if (int rc = peer_sync_all(ctx)) return rc;
+    if (p.y_end > p.y_begin) {
+        dim3 block(64, 4), grid((p.W + 63) / 64, (p.y_end - p.y_begin + 3) / 4);
+        if (peer_out) present_kernel<true><<<grid, block, 0, ctx->stream>>>(p);
+        else present_kernel<false><<<grid, block, 0, ctx->stream>>>(p);
+        VHR_CUDA_CHECK(cudaGetLastError());
+        ctx->launches++;
+    }
+    return gather ? peer_sync_all(ctx) : VHR_OK;      // every rank's rows have landed before anything on the output rank reads them
 }
 
 int launch_composition(vhr_context *ctx, int shadow_mode, int ao_mode, int reflection_mode) {
@@ -247,12 +315,29 @@ int launch_composition(vhr_context *ctx, int shadow_mode, int ao_mode, int refle
         return fail(VHR_ERR_INVALID, "composition: render output format %d", out->format);
     if (shadow_mode < 0 || shadow_mode > 2 || ao_mode < 0 || ao_mode > 2 || reflection_mode < 0 || reflection_mode > 2)
         return fail(VHR_ERR_INVALID, "composition: specialisation constants (%d, %d, %d)", shadow_mode, ao_mode, reflection_mode);
+    bool gather;
+    void *peer_out;
+    if (int rc = gather_target(ctx, out, "composition", gather, peer_out)) return rc;
+    typedef void (*Kernel)(const CompositionParams, const PerFrameData);
+    typedef void (*GatherKernel)(const CompositionGatherParams, const PerFrameData);
+#define VHR_COMP_ROW(S, A, G) {composition_kernel<S, A, 0, G>, composition_kernel<S, A, 1, G>, composition_kernel<S, A, 2, G>}
+#define VHR_COMP_TABLE(G) {{VHR_COMP_ROW(0, 0, G), VHR_COMP_ROW(0, 1, G), VHR_COMP_ROW(0, 2, G)}, \
+                           {VHR_COMP_ROW(1, 0, G), VHR_COMP_ROW(1, 1, G), VHR_COMP_ROW(1, 2, G)}, \
+                           {VHR_COMP_ROW(2, 0, G), VHR_COMP_ROW(2, 1, G), VHR_COMP_ROW(2, 2, G)}}
+    static const Kernel table[3][3][3] = VHR_COMP_TABLE(false);
+    static const GatherKernel gather_table[3][3][3] = VHR_COMP_TABLE(true);
+#undef VHR_COMP_TABLE
+#undef VHR_COMP_ROW
+    const Kernel single = table[shadow_mode][ao_mode][reflection_mode];
+    const GatherKernel both = gather_table[shadow_mode][ao_mode][reflection_mode];
+    if (gather)
+        if (int rc = load_pair(ctx, (shadow_mode * 3 + ao_mode) * 3 + reflection_mode, single, both)) return rc;
     if (int rc = make_writable(ctx, out, covers_image(ctx, out, out->width, out->height))) return rc;
-    CompositionParams p;
+    CompositionGatherParams p;      // its CompositionParams part is all the <false> instances take
     p.W = (int)out->width; p.H = (int)out->height;
     p.y_begin = std::max(0, ctx->opt.row_begin);
     p.y_end = ctx->opt.row_end < 0 ? p.H : std::min(p.H, ctx->opt.row_end);
-    if (p.y_end <= p.y_begin) return VHR_OK;
+    if (p.y_end <= p.y_begin && !gather) return VHR_OK;
     p.shadow_mode = shadow_mode; p.ao_mode = ao_mode; p.reflection_mode = reflection_mode;
     p.out_format = out->format;
     p.rt_is_rg16 = b[7]->format == VHR_FORMAT_R16G16_SFLOAT;
@@ -260,17 +345,18 @@ int launch_composition(vhr_context *ctx, int shadow_mode, int ao_mode, int refle
     p.albedo = (const uint32_t *)b[0]->ptr; p.normals = (const uint2 *)b[1]->ptr; p.motion = (const uint2 *)b[2]->ptr;
     p.depth = (const float *)b[3]->ptr; p.shadow_map = (const float *)b[4]->ptr; p.ssao = (const uint2 *)b[5]->ptr;
     p.ssr = (const uint2 *)b[6]->ptr; p.rt = b[7]->ptr; p.refl = (const uint2 *)b[8]->ptr; p.out = out->ptr;
-    dim3 block(64, 4), grid((p.W + 63) / 64, (p.y_end - p.y_begin + 3) / 4);
-    typedef void (*Kernel)(const CompositionParams, const PerFrameData);
-#define VHR_COMP_ROW(S, A) {composition_kernel<S, A, 0>, composition_kernel<S, A, 1>, composition_kernel<S, A, 2>}
-    static const Kernel table[3][3][3] = {{VHR_COMP_ROW(0, 0), VHR_COMP_ROW(0, 1), VHR_COMP_ROW(0, 2)},
-                                          {VHR_COMP_ROW(1, 0), VHR_COMP_ROW(1, 1), VHR_COMP_ROW(1, 2)},
-                                          {VHR_COMP_ROW(2, 0), VHR_COMP_ROW(2, 1), VHR_COMP_ROW(2, 2)}};
-#undef VHR_COMP_ROW
-    table[shadow_mode][ao_mode][reflection_mode]<<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
-    VHR_CUDA_CHECK(cudaGetLastError());
-    ctx->launches++;
-    return VHR_OK;
+    p.out_gather = peer_out;
+    // gathering: the output rank may still read the previous frame's output, and no earlier pass of this frame need have waited for it
+    if (gather)
+        if (int rc = peer_sync_all(ctx)) return rc;
+    if (p.y_end > p.y_begin) {
+        dim3 block(64, 4), grid((p.W + 63) / 64, (p.y_end - p.y_begin + 3) / 4);
+        if (peer_out) both<<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
+        else single<<<grid, block, 0, ctx->stream>>>(p, ctx->pfd);
+        VHR_CUDA_CHECK(cudaGetLastError());
+        ctx->launches++;
+    }
+    return gather ? peer_sync_all(ctx) : VHR_OK;      // every rank's rows have landed before anything on the output rank reads them
 }
 
 }  // namespace vhr

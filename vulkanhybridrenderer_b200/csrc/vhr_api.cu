@@ -868,6 +868,9 @@ int vhr_set_option(vhr_context *ctx, int option, int64_t value) {
             if (value < 0 || value > 3) return fail(VHR_ERR_INVALID, "atrous variant %lld", (long long)value);
             ctx->opt.atrous_variant = (int)value; return VHR_OK;
         case VHR_OPT_RAYTRACED_ALPHA_TEST: ctx->opt.raytraced_alpha_test = value != 0; return VHR_OK;
+        case VHR_OPT_OUTPUT_RANK:
+            if (value < -1 || value >= VHR_MAX_RANKS) return fail(VHR_ERR_INVALID, "output rank %lld out of [-1, %d]", (long long)value, VHR_MAX_RANKS - 1);
+            ctx->opt.output_rank = (int)value; return VHR_OK;
         case VHR_OPT_RAYGEN_VARIANT:
             if (value < 0 || value > 15 || value == 5) return fail(VHR_ERR_INVALID, "raygen variant %lld", (long long)value);
             ctx->opt.raygen_variant = (int)value; return VHR_OK;
@@ -902,6 +905,7 @@ int64_t vhr_get_option(vhr_context *ctx, int option) {
         case VHR_OPT_DEBUG_REFLECTION_T: return ctx->opt.debug_refl_t;
         case VHR_OPT_RAYGEN_VARIANT: return ctx->opt.raygen_variant;
         case VHR_OPT_RAYTRACED_ALPHA_TEST: return ctx->opt.raytraced_alpha_test;
+        case VHR_OPT_OUTPUT_RANK: return ctx->opt.output_rank;
     }
     return -1;
 }

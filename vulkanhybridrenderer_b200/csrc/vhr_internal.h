@@ -73,6 +73,7 @@ struct Options {
     int debug_refl_t = 0;        // 1: the ray pass also writes the reflection ray's hit distance (tests)
     int raytraced_alpha_test = 0; // the fully ray-traced path's use_anyhit_shader (raytraced_render_path.h:14)
     int raygen_variant = 0;      // 0 (default, fastest as measured): one thread per pixel, ray kinds in lock step; 1-4: see VHR_OPT_RAYGEN_VARIANT
+    int output_rank = -1;        // the rank whose render output the composition passes gather the partitioned frame into; -1 = off (VHR_OPT_OUTPUT_RANK)
 };
 
 // Row partition of one frame over the GPUs of a box (vhr_set_partition)

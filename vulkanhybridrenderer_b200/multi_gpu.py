@@ -172,8 +172,19 @@ def _gbuffer_names(path):
     return [g[k] for g in path.gsets for k in (HP.N_ALBEDO, HP.N_NORMALS, HP.N_MOTION, HP.N_DEPTH)]
 
 
+def _check_output_rank(ctxs, world, output_rank):
+    """output_rank must name a rank, and RENDER_OUTPUT must exist on every context before it can be exported or attached"""
+    from . import hybrid_path as HP
+    if not 0 <= output_rank < world:
+        raise ValueError(f"output_rank {output_rank} is not a rank of the partition (world {world})")
+    for ctx in ctxs:
+        if not _has_image(ctx, HP.N_RENDER_OUTPUT):
+            raise ValueError(f"output_rank: {HP.N_RENDER_OUTPUT!r} is not actualized on this context; create it before the partition "
+                             "(HybridRenderPath(..., composition=<format>), or ctx.actualize_image for the ray-traced path)")
+
+
 def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False,
-                          exchange_shadow_map=False):
+                          exchange_shadow_map=False, output_rank=None):
     """Exports this rank's exchanged images, attaches everybody else's, installs the row partition on `ctx`.
 
     Exchanged images: the ray pass outputs (every rank stores into every owner's), the two integrated ping-pong images and
@@ -182,15 +193,20 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
     exchange_gbuffer: also the four images of every G-buffer set, attached for all ranks, so that `HybridRenderPath.gbuffer_pass`
     runs partitioned (every rank traces its rows and stores them into every rank's G-buffer): the frame is driven from a camera.
     exchange_shadow_map: also the "Shadow Map", attached for all ranks, so that `HybridRenderPath.shadow_map_pass` runs partitioned
-    (every rank rasterises its 8-row blocks of the map and stores them into every rank's map)."""
+    (every rank rasterises its 8-row blocks of the map and stores them into every rank's map).
+    output_rank: also rank `output_rank`'s RENDER_OUTPUT, attached on every other rank, and VHR_OPT_OUTPUT_RANK on every rank, so that
+    the composition draws gather the whole frame into that rank's RENDER_OUTPUT. RENDER_OUTPUT must already exist on every rank."""
     import torch.distributed as dist
-    from . import hybrid_path as HP
+    from . import capi, hybrid_path as HP
+    if output_rank is not None:
+        _check_output_rank([ctx], world, output_rank)
     pc = path.pc
     mine = {"sync": ctx.sync_export_ipc(), "rt": [], "integ": [], "moments": None}
     for rt_name, refl_name in path.rt_sets:
         mine["rt"].append((ctx.image_export_ipc(rt_name), ctx.image_export_ipc(refl_name)))
     mine["gbuffer"] = [ctx.image_export_ipc(n) for n in _gbuffer_names(path)] if exchange_gbuffer else []
     mine["shadow_map"] = ctx.image_export_ipc(HP.N_SHADOW_MAP) if exchange_shadow_map else None
+    mine["render_output"] = ctx.image_export_ipc(HP.N_RENDER_OUTPUT) if output_rank == rank else None
     for slot in pc["integrated_shadow_and_ao"]:
         mine["integ"].append((int(slot), ctx.storage_image_export_ipc(int(slot))[0]))
     mslot = int(pc["shadow_and_ao_moments_history"])
@@ -211,6 +227,8 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
             ctx.image_attach_peer(name, r, h)
         if other["shadow_map"] is not None:
             ctx.image_attach_peer(HP.N_SHADOW_MAP, r, other["shadow_map"])
+        if other["render_output"] is not None:
+            ctx.image_attach_peer(HP.N_RENDER_OUTPUT, r, other["render_output"])
         if abs(r - rank) == 1:                       # halos only ever go to the two neighbours
             for (slot, _), (_, h) in zip(mine["integ"], other["integ"]):
                 ctx.storage_image_attach_peer(slot, r, h)
@@ -219,19 +237,24 @@ def setup_fused_partition(ctx, path, world, rank, group=None, motion_halo=8, ray
                 ctx.image_attach_peer("Screen Space Ambient Occlusion Raw", r, other["ssao_raw"])
     bands = [band_rows(path.H, world, r)[0] for r in range(world)] + [path.H]
     ctx.set_partition(world, rank, bands, ray_block_rows=ray_block_rows, motion_halo=motion_halo)
+    if output_rank is not None:
+        ctx.set_option(capi.OPT_OUTPUT_RANK, output_rank)
     dist.barrier(group=group)                        # nobody starts storing into a peer that has not attached yet
     return bands
 
 
-def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False, exchange_shadow_map=False):
+def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8, exchange_gbuffer=False, exchange_shadow_map=False,
+                                    output_rank=None):
     """The same partition for ranks that live in ONE process (one context per rank, all driven by this thread): peers are
     attached by plain device pointer. With all contexts on one GPU this exercises the whole fused path — interleaved ray
     blocks, halo pushes, flag-word ordering between the streams — on a single-GPU box (tests/test_partition_gpu.py).
-    exchange_gbuffer, exchange_shadow_map: as for setup_fused_partition."""
+    exchange_gbuffer, exchange_shadow_map, output_rank: as for setup_fused_partition."""
     from . import capi, hybrid_path as HP
     L = capi.lib()
     world = len(ctxs)
     H = paths[0].H
+    if output_rank is not None:
+        _check_output_rank(ctxs, world, output_rank)
     for r, (ctx, path) in enumerate(zip(ctxs, paths)):
         for q, (octx, opath) in enumerate(zip(ctxs, paths)):
             if q == r:
@@ -245,6 +268,8 @@ def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8
                     capi._check(L.vhr_image_attach_peer_pointer(ctx._h, name.encode(), q, octx.image_info(oname)[0]))
             if exchange_shadow_map:
                 capi._check(L.vhr_image_attach_peer_pointer(ctx._h, HP.N_SHADOW_MAP.encode(), q, octx.image_info(HP.N_SHADOW_MAP)[0]))
+            if q == output_rank:
+                capi._check(L.vhr_image_attach_peer_pointer(ctx._h, HP.N_RENDER_OUTPUT.encode(), q, octx.image_info(HP.N_RENDER_OUTPUT)[0]))
             if abs(q - r) == 1:
                 for slot, oslot in zip(path.pc["integrated_shadow_and_ao"], opath.pc["integrated_shadow_and_ao"]):
                     capi._check(L.vhr_storage_image_attach_peer_pointer(ctx._h, int(slot), q, octx.storage_image_info(int(oslot))[0], None))
@@ -258,6 +283,8 @@ def setup_fused_partition_inprocess(ctxs, paths, motion_halo=8, ray_block_rows=8
     bands = [band_rows(H, world, r)[0] for r in range(world)] + [H]
     for r, ctx in enumerate(ctxs):
         ctx.set_partition(world, r, bands, ray_block_rows=ray_block_rows, motion_halo=motion_halo)
+        if output_rank is not None:
+            ctx.set_option(capi.OPT_OUTPUT_RANK, output_rank)
     return bands
 
 
