@@ -355,6 +355,42 @@ int vhr_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int any_
  * outputs hit distances (its payloads are 0/1 and radiance); this exists for the hit-distance parity check. */
 int vhr_debug_download_reflection_t(vhr_context *ctx, float *host, size_t bytes);
 
+/* Test entry point: runs the per-hit shading code of the passes on hits the caller chooses, so that tests can hold it to a reference
+ * on identical hits (the traversal, which decides where a ray hits, is not involved). Record i names a hit by geometry index g
+ * (the flat primitive index of vhr_update_geometry), primitive id pid (triangle pid of that primitive) and the barycentrics (u, v) of
+ * its vertices 1 and 2, as vhr_trace_explicit returns them. The code runs against the context's state: geometry, normal matrices,
+ * the textures of vhr_upload_texture_from_data with their samplers, and the per-frame constants. `out` receives
+ * VHR_SHADE_OUT_WORDS 32-bit words per record; words a kind does not write are 0.
+ *   VHR_SHADE_TEXTURE           texture(textures[g], (u, v)) at LOD 0 with the slot's sampler (pid, x, y unused): RGBA as 4 floats
+ *   VHR_SHADE_REFLECTION        the reflection ray's closest-hit shading (reflection_hit.rchit): RGBA radiance as 4 floats, before
+ *                               the RGBA16F store of the ray pass
+ *   VHR_SHADE_GBUFFER           the G-buffer pass's texel for a primary hit seen through pixel (x, y): the albedo word (BGRA8), the two
+ *                               normals / object-id words (RGBA16F), the two motion / metallic-roughness words (RGBA16F), depth (D32)
+ *   VHR_SHADE_GBUFFER_ALPHA     the G-buffer pass's any-hit test (gbuf.frag's discards): 1 = the candidate counts, 0 = discarded
+ *   VHR_SHADE_RAYTRACED[_ALPHA] the fully ray-traced path's closest-hit shading (the opaque / the alpha-tested pipeline): the output
+ *                               word (BGRA8) when the shadow ray is not occluded, the word when it is, the shadow ray's origin (3 floats)
+ *   VHR_SHADE_ANYHIT_ALPHA      the alpha-tested pipeline's any-hit test (shadow_anyhit.rahit): 1 = the candidate counts, 0 = ignored
+ * Every record is checked before anything runs: g < the number of primitives and pid < its index_count / 3 (a texture slot in use for
+ * VHR_SHADE_TEXTURE); an unknown kind, a NULL array or an invalid record is VHR_ERR_INVALID. VHR_ERR_STATE without per-frame constants
+ * or, for the kinds that shade a hit, without geometry; VHR_ERR_CUDA on a VHR_DEVICE_NONE context. Synchronous. */
+typedef struct vhr_shade_record {
+    uint32_t g;       /* geometry index (VHR_SHADE_TEXTURE: texture slot) */
+    uint32_t pid;     /* primitive id within the geometry */
+    float u, v;       /* barycentrics of vertices 1 and 2 (VHR_SHADE_TEXTURE: texture coordinates s, t) */
+    int32_t x, y;     /* pixel (VHR_SHADE_GBUFFER only) */
+} vhr_shade_record;
+enum {
+    VHR_SHADE_TEXTURE = 0,
+    VHR_SHADE_REFLECTION = 1,
+    VHR_SHADE_GBUFFER = 2,
+    VHR_SHADE_GBUFFER_ALPHA = 3,
+    VHR_SHADE_RAYTRACED = 4,
+    VHR_SHADE_RAYTRACED_ALPHA = 5,
+    VHR_SHADE_ANYHIT_ALPHA = 6
+};
+#define VHR_SHADE_OUT_WORDS 8
+int vhr_debug_shade_hits(vhr_context *ctx, int kind, const vhr_shade_record *records, uint32_t n, uint32_t *out);
+
 /* G-buffer producer as a CUDA primary-ray pass (stand-in for the rasterised "G-Buffer Pass",
  * hybrid_render_path.cpp:13-56; encodings of gbuf.frag:33,43,46-58). Bound images: 0 albedo (BGRA8), 1 normals/ids,
  * 2 motion/metallic-roughness, 3 depth.

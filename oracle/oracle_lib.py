@@ -89,6 +89,8 @@ def _declare(L):
     L.vo_raygen_pixel_rays.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp]
     L.vo_brute_force.argtypes = [vp, vp, vp, C.c_float, C.c_float, vp]
     L.vo_gbuffer.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp, vp, vp, vp]
+    L.vo_shade_hits.restype = C.c_int
+    L.vo_shade_hits.argtypes = [vp, vp, C.c_int, vp, C.c_uint32, vp]
 
 
 def set_num_threads(n=0):
@@ -262,6 +264,15 @@ class OracleScene:
         if want_ids:
             g["ids"] = ids
         return g
+
+    def shade_hits(self, pfd, kind, records):
+        """The per-hit code of the passes on the given hits, kinds and output words as vhr_debug_shade_hits (Context.shade_hits):
+        [n, T.SHADE_OUT_WORDS] uint32."""
+        rec = np.ascontiguousarray(records, T.ShadeRecord).reshape(-1)
+        out = np.zeros((len(rec), T.SHADE_OUT_WORDS), np.uint32)
+        if lib().vo_shade_hits(self._s, _p(pfd), int(kind), _p(rec), len(rec), _p(out)) != 0:
+            raise ValueError("vo_shade_hits: unknown kind or a record naming a texture / triangle that does not exist")
+        return out
 
     def raytraced(self, pfd, W, H, alpha_test=False):
         """The fully ray-traced render path's "Raytracing Pass": [H, W, 4] uint8 B8G8R8A8_UNORM "RaytracedOutput"."""

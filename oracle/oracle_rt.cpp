@@ -8,6 +8,7 @@
 //                        reflection_miss.rmiss:6-8, reflection_hit.rchit:10-72)
 //   vo_gbuffer        <- data/shaders/hybrid_render_path/gbuf.vert:19-28, gbuf.frag:17-59 and the clear values
 //                        of hybrid_render_path.cpp:16-19 (scaffolding: primary rays stand in for the rasteriser)
+//   vo_shade_hits     <- the per-hit code of the passes above and of vo_raytraced on hits the caller gives (tests)
 //
 // The reference's BVH build, traversal and ray/triangle test live inside the Vulkan driver
 // (vkCmdBuildAccelerationStructuresKHR / traceRayEXT — third-party, unversioned; SURVEY §8c). They are
@@ -19,6 +20,8 @@
 #include <algorithm>
 #include <atomic>
 #include <cfloat>
+#include <climits>
+#include <cstring>
 #include <vector>
 #ifdef _OPENMP
 #include <omp.h>
@@ -334,9 +337,8 @@ bool trace_closest(const Scene &s, vec3 o, vec3 d, float tmin, float tmax, Hit &
     return trace_closest_filtered(s, o, d, tmin, tmax, hit, [](uint32_t, double, double) { return true; });
 }
 
-// reflection_hit.rchit:10-72
-vec4 reflection_hit(const Scene &s, const PerFrameData &pfd, const Hit &hit) {
-    uint32_t g = s.tri_geom[hit.tri], pid = s.tri_prim[hit.tri];
+// reflection_hit.rchit:10-72 for triangle pid of geometry g at the barycentrics (hx, hy) of vertices 1 and 2
+vec4 reflection_hit(const Scene &s, const PerFrameData &pfd, uint32_t g, uint32_t pid, float hx, float hy) {
     const Primitive &prim = s.primitives[g];
     uint32_t i0 = s.indices[prim.index_offset + 3 * pid + 0];
     uint32_t i1 = s.indices[prim.index_offset + 3 * pid + 1];
@@ -344,7 +346,6 @@ vec4 reflection_hit(const Scene &s, const PerFrameData &pfd, const Hit &hit) {
     const Vertex &v0 = s.vertices[prim.vertex_offset + i0];
     const Vertex &v1 = s.vertices[prim.vertex_offset + i1];
     const Vertex &v2 = s.vertices[prim.vertex_offset + i2];
-    float hx = (float)hit.u, hy = (float)hit.v;
     float b0 = 1.0f - hx - hy, b1 = hx, b2 = hy;
     vec3 normal = v3(v0.normal[0], v0.normal[1], v0.normal[2]) * b0 + v3(v1.normal[0], v1.normal[1], v1.normal[2]) * b1 +
                   v3(v2.normal[0], v2.normal[1], v2.normal[2]) * b2;
@@ -386,6 +387,158 @@ vec4 reflection_hit(const Scene &s, const PerFrameData &pfd, const Hit &hit) {
     float ndl = gl_max(dot(N, L), 0.0f);
     vec3 lighting = ambient + (diffuse + specular) * ndl * li * lc;
     return vec4{lighting.x, lighting.y, lighting.z, 1.0f};
+}
+
+// gbuf.frag:19-32, the any-hit stage of the primary ray: a fragment failing the alpha-mask test, or with alpha exactly 0, is
+// discarded. (c1, c2) = barycentrics of vertices 1 and 2.
+bool gbuffer_alpha_test(const Scene &s, uint32_t g, uint32_t k, float c1, float c2) {
+    const Primitive &pr = s.primitives[g];
+    float alpha = pr.material.base_color[3];
+    if (has_texture(s, pr.material.base_color_texture)) {
+        const Vertex &a0 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 0]];
+        const Vertex &a1 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 1]];
+        const Vertex &a2 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 2]];
+        float c0 = 1.0f - c1 - c2;
+        vec2 uvt = {a0.uv0[0] * c0 + a1.uv0[0] * c1 + a2.uv0[0] * c2, a0.uv0[1] * c0 + a1.uv0[1] * c1 + a2.uv0[1] * c2};
+        alpha = sample_texture(s, pr.material.base_color_texture, uvt).w;
+    }
+    if (pr.material.alpha_mask == 1 && alpha < pr.material.alpha_cutoff) return false;
+    return alpha != 0.0f;
+}
+
+// shadow_anyhit.rahit:22-26 (the shader samples textures[base_color_texture] unconditionally; index -1 counts as opaque here)
+bool rahit_alpha_test(const Scene &s, uint32_t g, uint32_t k, float c1, float c2) {
+    const Primitive &pr = s.primitives[g];
+    if (pr.material.alpha_mask != 1 || !has_texture(s, pr.material.base_color_texture)) return true;
+    const Vertex &a0 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 0]];
+    const Vertex &a1 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 1]];
+    const Vertex &a2 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 2]];
+    float c0 = 1.0f - c1 - c2;
+    vec2 uvt = {a0.uv0[0] * c0 + a1.uv0[0] * c1 + a2.uv0[0] * c2, a0.uv0[1] * c0 + a1.uv0[1] * c1 + a2.uv0[1] * c2};
+    return !(sample_texture(s, pr.material.base_color_texture, uvt).w < pr.material.alpha_cutoff);
+}
+
+// closesthit.rchit:11-41 for one hit: the albedo, the shading normal N and the world-space hit point (the shadow ray's origin)
+struct RaytracedHit { vec3 albedo, N, position; };
+RaytracedHit raytraced_hit(const Scene &s, uint32_t g, uint32_t pid, float b1, float b2) {
+    const Primitive &prim = s.primitives[g];
+    const Vertex &v0 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
+    const Vertex &v1 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
+    const Vertex &v2 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
+    float b0 = 1.0f - b1 - b2;
+    vec2 tuv = {v0.uv0[0] * b0 + v1.uv0[0] * b1 + v2.uv0[0] * b2, v0.uv0[1] * b0 + v1.uv0[1] * b1 + v2.uv0[1] * b2};
+    vec3 normal = v3(v0.normal[0], v0.normal[1], v0.normal[2]) * b0 + v3(v1.normal[0], v1.normal[1], v1.normal[2]) * b1 +
+                  v3(v2.normal[0], v2.normal[1], v2.normal[2]) * b2;
+    vec3 pobj = v3(v0.pos[0], v0.pos[1], v0.pos[2]) * b0 + v3(v1.pos[0], v1.pos[1], v1.pos[2]) * b1 +
+                v3(v2.pos[0], v2.pos[1], v2.pos[2]) * b2;
+    vec4 pw = mul44(prim.transform, vec4{pobj.x, pobj.y, pobj.z, 1.0f});
+    RaytracedHit r;
+    r.position = v3(pw.x, pw.y, pw.z);
+    r.albedo = v3(prim.material.base_color[0], prim.material.base_color[1], prim.material.base_color[2]);
+    if (has_texture(s, prim.material.base_color_texture)) {
+        vec4 c = sample_texture(s, prim.material.base_color_texture, tuv);
+        r.albedo = v3(c.x, c.y, c.z);
+    }
+    r.N = normal;
+    if (has_texture(s, prim.material.normal_map)) {                                       // closesthit.rchit:35-41
+        vec3 tan3 = v3(v0.tangent[0], v0.tangent[1], v0.tangent[2]) * b0 + v3(v1.tangent[0], v1.tangent[1], v1.tangent[2]) * b1 +
+                    v3(v2.tangent[0], v2.tangent[1], v2.tangent[2]) * b2;
+        float tw = v0.tangent[3] * b0 + v1.tangent[3] * b1 + v2.tangent[3] * b2;
+        vec4 c = sample_texture(s, prim.material.normal_map, tuv);
+        vec3 tsn = normalize(v3(c.x * 2.0f - 1.0f, c.y * 2.0f - 1.0f, c.z * 2.0f - 1.0f));
+        vec3 bitangent = cross(tsn, tan3) * tw;
+        vec3 tangent = normalize(tan3 - normal * dot(tan3, normal));
+        r.N = tangent * tsn.x + bitangent * tsn.y + normal * tsn.z;
+    }
+    return r;
+}
+
+// closesthit.rchit:43-57 / closesthit_test_alpha.rchit:37-50: the payload of a shaded hit given the shadow ray's answer
+vec4 raytraced_color(const PerFrameData &pfd, int alpha_test, vec3 albedo, vec3 N, bool occluded) {
+    vec3 light_dir = -v3(pfd.directional_light.direction[0], pfd.directional_light.direction[1], pfd.directional_light.direction[2]);
+    vec3 lc = v3(pfd.directional_light.color[0], pfd.directional_light.color[1], pfd.directional_light.color[2]);
+    vec3 li = v3(pfd.directional_light.intensity[0], pfd.directional_light.intensity[1], pfd.directional_light.intensity[2]);
+    vec3 albedo_lighting = albedo * (alpha_test ? 0.2f : PI_INVERSE_F);
+    vec3 c = albedo_lighting;
+    if (!occluded) {
+        float ndl = gl_max(dot(N, light_dir), 0.0f);
+        vec3 lit = alpha_test ? (albedo * ndl) * lc : ((albedo * ndl) * li) * lc;
+        c = albedo_lighting + lit;
+    }
+    return vec4{c.x, c.y, c.z, 1.0f};
+}
+
+// imageStore to a B8G8R8A8_UNORM image: float -> UNORM8 (NaN -> 0), B first
+inline void store_bgra8(uint8_t *o, vec4 payload) {
+    auto q = [](float f) { f = (f == f) ? std::min(std::max(f, 0.0f), 1.0f) : 0.0f; return (uint8_t)std::lrintf(f * 255.0f); };
+    o[0] = q(payload.z); o[1] = q(payload.y); o[2] = q(payload.x); o[3] = q(payload.w);
+}
+
+// gl_FragCoord.xy * display_size_inverse of pixel (x, y)
+inline vec2 gbuffer_pixel_uv(const PerFrameData &pfd, int x, int y) {
+    return vec2{((float)x + 0.5f) * pfd.display_size_inverse[0], ((float)y + 0.5f) * pfd.display_size_inverse[1]};
+}
+
+// gbuf.frag:33-58 for a primary hit seen through the pixel at uv (gbuffer_pixel_uv): albedo BGRA8 (albedo4 may be NULL),
+// normals / object id RGBA16F, motion / metallic-roughness RGBA16F, depth D32
+void gbuffer_hit(const Scene &s, const PerFrameData &pfd, uint32_t g, uint32_t pid, float b1, float b2, vec2 uv, uint8_t *albedo_out,
+                 uint16_t *normals_out, uint16_t *motion_out, float *depth_out) {
+    const Primitive &prim = s.primitives[g];
+    const Vertex &v0 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
+    const Vertex &v1 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
+    const Vertex &v2 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
+    float b0 = 1.0f - b1 - b2;
+    vec3 nobj = v3(v0.normal[0], v0.normal[1], v0.normal[2]) * b0 + v3(v1.normal[0], v1.normal[1], v1.normal[2]) * b1 +
+                v3(v2.normal[0], v2.normal[1], v2.normal[2]) * b2;
+    vec3 pobj = v3(v0.pos[0], v0.pos[1], v0.pos[2]) * b0 + v3(v1.pos[0], v1.pos[1], v1.pos[2]) * b1 +
+                v3(v2.pos[0], v2.pos[1], v2.pos[2]) * b2;
+    const Material &mat = prim.material;
+    vec2 tuv = {v0.uv0[0] * b0 + v1.uv0[0] * b1 + v2.uv0[0] * b2, v0.uv0[1] * b0 + v1.uv0[1] * b1 + v2.uv0[1] * b2};
+    vec4 albedo4 = {mat.base_color[0], mat.base_color[1], mat.base_color[2], mat.base_color[3]};
+    if (has_texture(s, mat.base_color_texture)) albedo4 = sample_texture(s, mat.base_color_texture, tuv);       // gbuf.frag:20-26
+    if (has_texture(s, mat.normal_map)) {                                                                     // gbuf.frag:35-41
+        vec4 c = sample_texture(s, mat.normal_map, tuv);
+        vec3 tsn = normalize(v3(c.x * 2.0f - 1.0f, c.y * 2.0f - 1.0f, c.z * 2.0f - 1.0f));
+        vec3 tan3 = v3(v0.tangent[0], v0.tangent[1], v0.tangent[2]) * b0 + v3(v1.tangent[0], v1.tangent[1], v1.tangent[2]) * b1 +
+                    v3(v2.tangent[0], v2.tangent[1], v2.tangent[2]) * b2;
+        float tw = v0.tangent[3] * b0 + v1.tangent[3] * b1 + v2.tangent[3] * b2;
+        vec3 bitangent = cross(tsn, tan3) * tw;
+        vec3 tangent = normalize(tan3 - nobj * dot(tan3, nobj));
+        nobj = tangent * tsn.x + bitangent * tsn.y + nobj * tsn.z;
+    }
+    float metallic = mat.metallic_factor, roughness = mat.roughness_factor;
+    if (has_texture(s, mat.metallic_roughness_texture)) {                                                     // gbuf.frag:52-56
+        vec4 c = sample_texture(s, mat.metallic_roughness_texture, tuv);
+        metallic *= c.y;
+        roughness *= c.z;
+    }
+    // normal_matrix = inverseTranspose(mat3(transform)) (hybrid_render_path.cpp:45) = cofactor(M) / det(M)
+    const float *m = prim.transform;
+    double a00 = m[0], a10 = m[1], a20 = m[2], a01 = m[4], a11 = m[5], a21 = m[6], a02 = m[8], a12 = m[9], a22 = m[10];
+    double c00 = a11 * a22 - a21 * a12, c01 = -(a10 * a22 - a20 * a12), c02 = a10 * a21 - a20 * a11;
+    double c10 = -(a01 * a22 - a21 * a02), c11 = a00 * a22 - a20 * a02, c12 = -(a00 * a21 - a20 * a01);
+    double c20 = a01 * a12 - a11 * a02, c21 = -(a00 * a12 - a10 * a02), c22 = a00 * a11 - a10 * a01;
+    double det = a00 * c00 + a01 * c01 + a02 * c02;
+    // (M^-T)[r][c] = cof[r][c] / det, with cof indexed [row][col] of M (a_rc = m[c*4+r])
+    float nm[9] = {(float)(c00 / det), (float)(c10 / det), (float)(c20 / det),    // column 0: rows 0..2
+                   (float)(c01 / det), (float)(c11 / det), (float)(c21 / det),    // column 1
+                   (float)(c02 / det), (float)(c12 / det), (float)(c22 / det)};   // column 2
+    vec3 nw = {nm[0] * nobj.x + nm[3] * nobj.y + nm[6] * nobj.z,
+               nm[1] * nobj.x + nm[4] * nobj.y + nm[7] * nobj.z,
+               nm[2] * nobj.x + nm[5] * nobj.y + nm[8] * nobj.z};
+    nw = normalize(nw);
+    vec4 pw = mul44(prim.transform, vec4{pobj.x, pobj.y, pobj.z, 1.0f});
+    vec4 clip = mul44(pfd.camera_proj, mul44(pfd.camera_view, pw));
+    vec4 pclip = mul44(pfd.camera_proj_prev_frame, mul44(pfd.camera_view_prev_frame, pw));
+    vec2 cur_ndc = uv;   // gl_FragCoord.xy * display_size_inverse
+    vec2 prev_ndc = {(pclip.x / pclip.w) * 0.5f + 0.5f, (pclip.y / pclip.w) * 0.5f + 0.5f};
+    if (albedo_out) {
+        auto q = [](float f) { f = (f == f) ? std::min(std::max(f, 0.0f), 1.0f) : 0.0f; return (uint8_t)std::lrintf(f * 255.0f); };   // NaN -> 0
+        albedo_out[0] = q(albedo4.z); albedo_out[1] = q(albedo4.y); albedo_out[2] = q(albedo4.x); albedo_out[3] = q(albedo4.w);
+    }
+    store_rgba16f(normals_out, 1, 0, 0, vec4{nw.x, nw.y, nw.z, (float)g});
+    store_rgba16f(motion_out, 1, 0, 0, vec4{cur_ndc.x - prev_ndc.x, cur_ndc.y - prev_ndc.y, metallic, roughness});
+    *depth_out = clip.z / clip.w;
 }
 
 }  // namespace
@@ -571,7 +724,7 @@ void vo_raygen(const vo_scene *s_, const PerFrameData *pfd_, int W, int H, int y
                 Hit h;
                 vec4 payload = {0, 0, 0, 0};
                 float t = -1.0f;
-                if (trace_closest(s, origin, refl, 0.01f, 10000.0f, h)) { payload = reflection_hit(s, pfd, h); t = (float)h.t; }
+                if (trace_closest(s, origin, refl, 0.01f, 10000.0f, h)) { payload = reflection_hit(s, pfd, s.tri_geom[h.tri], s.tri_prim[h.tri], (float)h.u, (float)h.v); t = (float)h.t; }
                 rays++;
                 if (reflections) store_rgba16f(reflections, W, x, y, payload);
                 if (refl_t) refl_t[(size_t)y * W + x] = t;
@@ -659,18 +812,7 @@ void vo_brute_force(const vo_scene *s_, const float *o_, const float *d_, float 
 void vo_raytraced(const vo_scene *s_, const PerFrameData *pfd_, int W, int H, int alpha_test, uint8_t *out_bgra8) {
     const Scene &s = *reinterpret_cast<const Scene *>(s_);
     const PerFrameData &pfd = *pfd_;
-    // shadow_anyhit.rahit:22-26 (the shader samples textures[base_color_texture] unconditionally; index -1 counts as opaque here)
-    auto rahit = [&](uint32_t tri, double hu, double hv) {
-        const Primitive &pr = s.primitives[s.tri_geom[tri]];
-        if (pr.material.alpha_mask != 1 || !has_texture(s, pr.material.base_color_texture)) return true;
-        uint32_t k = s.tri_prim[tri];
-        const Vertex &a0 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 0]];
-        const Vertex &a1 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 1]];
-        const Vertex &a2 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 2]];
-        float c1 = (float)hu, c2 = (float)hv, c0 = 1.0f - c1 - c2;
-        vec2 uvt = {a0.uv0[0] * c0 + a1.uv0[0] * c1 + a2.uv0[0] * c2, a0.uv0[1] * c0 + a1.uv0[1] * c1 + a2.uv0[1] * c2};
-        return !(sample_texture(s, pr.material.base_color_texture, uvt).w < pr.material.alpha_cutoff);
-    };
+    auto rahit = [&](uint32_t tri, double hu, double hv) { return rahit_alpha_test(s, s.tri_geom[tri], s.tri_prim[tri], (float)hu, (float)hv); };
     auto opaque = [](uint32_t, double, double) { return true; };
 #pragma omp parallel for schedule(dynamic, 1)
     for (int y = 0; y < H; ++y) {
@@ -686,54 +828,59 @@ void vo_raytraced(const vo_scene *s_, const PerFrameData *pfd_, int W, int H, in
             bool hit = alpha_test ? trace_closest_filtered(s, v3(origin.x, origin.y, origin.z), v3(direction.x, direction.y, direction.z), 0.1f, 10000.0f, h, rahit)
                                   : trace_closest_filtered(s, v3(origin.x, origin.y, origin.z), v3(direction.x, direction.y, direction.z), 0.1f, 10000.0f, h, opaque);
             if (hit) {
-                uint32_t g = s.tri_geom[h.tri], pid = s.tri_prim[h.tri];
-                const Primitive &prim = s.primitives[g];
-                const Vertex &v0 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
-                const Vertex &v1 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
-                const Vertex &v2 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
-                float b1 = (float)h.u, b2 = (float)h.v, b0 = 1.0f - b1 - b2;
-                vec2 tuv = {v0.uv0[0] * b0 + v1.uv0[0] * b1 + v2.uv0[0] * b2, v0.uv0[1] * b0 + v1.uv0[1] * b1 + v2.uv0[1] * b2};
-                vec3 normal = v3(v0.normal[0], v0.normal[1], v0.normal[2]) * b0 + v3(v1.normal[0], v1.normal[1], v1.normal[2]) * b1 +
-                              v3(v2.normal[0], v2.normal[1], v2.normal[2]) * b2;
-                vec3 pobj = v3(v0.pos[0], v0.pos[1], v0.pos[2]) * b0 + v3(v1.pos[0], v1.pos[1], v1.pos[2]) * b1 +
-                            v3(v2.pos[0], v2.pos[1], v2.pos[2]) * b2;
-                vec4 pw = mul44(prim.transform, vec4{pobj.x, pobj.y, pobj.z, 1.0f});
-                vec3 position = v3(pw.x, pw.y, pw.z);
-                vec3 albedo = v3(prim.material.base_color[0], prim.material.base_color[1], prim.material.base_color[2]);
-                if (has_texture(s, prim.material.base_color_texture)) {
-                    vec4 c = sample_texture(s, prim.material.base_color_texture, tuv);
-                    albedo = v3(c.x, c.y, c.z);
-                }
-                vec3 N = normal;
-                if (has_texture(s, prim.material.normal_map)) {                                   // closesthit.rchit:35-41
-                    vec3 tan3 = v3(v0.tangent[0], v0.tangent[1], v0.tangent[2]) * b0 + v3(v1.tangent[0], v1.tangent[1], v1.tangent[2]) * b1 +
-                                v3(v2.tangent[0], v2.tangent[1], v2.tangent[2]) * b2;
-                    float tw = v0.tangent[3] * b0 + v1.tangent[3] * b1 + v2.tangent[3] * b2;
-                    vec4 c = sample_texture(s, prim.material.normal_map, tuv);
-                    vec3 tsn = normalize(v3(c.x * 2.0f - 1.0f, c.y * 2.0f - 1.0f, c.z * 2.0f - 1.0f));
-                    vec3 bitangent = cross(tsn, tan3) * tw;
-                    vec3 tangent = normalize(tan3 - normal * dot(tan3, normal));
-                    N = tangent * tsn.x + bitangent * tsn.y + normal * tsn.z;
-                }
+                RaytracedHit r = raytraced_hit(s, s.tri_geom[h.tri], s.tri_prim[h.tri], (float)h.u, (float)h.v);
                 vec3 light_dir = -v3(pfd.directional_light.direction[0], pfd.directional_light.direction[1], pfd.directional_light.direction[2]);
-                vec3 lc = v3(pfd.directional_light.color[0], pfd.directional_light.color[1], pfd.directional_light.color[2]);
-                vec3 li = v3(pfd.directional_light.intensity[0], pfd.directional_light.intensity[1], pfd.directional_light.intensity[2]);
                 Hit sh;
-                bool occluded = alpha_test ? trace_closest_filtered(s, position, light_dir, 0.1f, 10000.0f, sh, rahit) : trace_any(s, position, light_dir, 0.1f, 10000.0f);
-                vec3 albedo_lighting = albedo * (alpha_test ? 0.2f : PI_INVERSE_F);
-                vec3 c = albedo_lighting;
-                if (!occluded) {
-                    float ndl = gl_max(dot(N, light_dir), 0.0f);
-                    vec3 lit = alpha_test ? (albedo * ndl) * lc : ((albedo * ndl) * li) * lc;
-                    c = albedo_lighting + lit;
-                }
-                payload = vec4{c.x, c.y, c.z, 1.0f};
+                bool occluded = alpha_test ? trace_closest_filtered(s, r.position, light_dir, 0.1f, 10000.0f, sh, rahit) : trace_any(s, r.position, light_dir, 0.1f, 10000.0f);
+                payload = raytraced_color(pfd, alpha_test, r.albedo, r.N, occluded);
             }
-            auto q = [](float f) { f = (f == f) ? std::min(std::max(f, 0.0f), 1.0f) : 0.0f; return (uint8_t)std::lrintf(f * 255.0f); };
-            uint8_t *o = out_bgra8 + ((size_t)y * W + x) * 4;
-            o[0] = q(payload.z); o[1] = q(payload.y); o[2] = q(payload.x); o[3] = q(payload.w);
+            store_bgra8(out_bgra8 + ((size_t)y * W + x) * 4, payload);
         }
     }
+}
+
+// The per-hit code of the passes on hits the caller chooses, kinds and outputs as vhr_debug_shade_hits (include/vhr_b200.h): record i =
+// (g, pid, u, v, x, y) as uint32 g, uint32 pid, float u, float v, int32 x, int32 y; 8 words out per record, unwritten words 0. Returns 0,
+// or -1 (nothing written) for an unknown kind or a record naming a texture, geometry or triangle that does not exist.
+struct ShadeRecord { uint32_t g, pid; float u, v; int32_t x, y; };
+int vo_shade_hits(const vo_scene *s_, const PerFrameData *pfd_, int kind, const ShadeRecord *rec, uint32_t n, uint32_t *out) {
+    const Scene &s = *reinterpret_cast<const Scene *>(s_);
+    const PerFrameData &pfd = *pfd_;
+    if (kind < 0 || kind > 6) return -1;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (kind == 0 ? !has_texture(s, (int)std::min<uint32_t>(rec[i].g, INT32_MAX))
+                      : rec[i].g >= s.primitives.size() || rec[i].pid >= s.primitives[rec[i].g].index_count / 3)
+            return -1;
+    }
+    std::memset(out, 0, (size_t)n * 8 * sizeof(uint32_t));
+#pragma omp parallel for schedule(static)
+    for (long long i = 0; i < (long long)n; ++i) {
+        const ShadeRecord &r = rec[i];
+        uint32_t *o = out + 8 * i;
+        auto put4 = [&](vec4 c) { std::memcpy(o, &c, 16); };
+        switch (kind) {
+            case 0: put4(sample_texture(s, (int)r.g, vec2{r.u, r.v})); break;
+            case 1: put4(reflection_hit(s, pfd, r.g, r.pid, r.u, r.v)); break;
+            case 2: {
+                uint16_t nrm[4], mot[4];
+                float depth;
+                gbuffer_hit(s, pfd, r.g, r.pid, r.u, r.v, gbuffer_pixel_uv(pfd, r.x, r.y), reinterpret_cast<uint8_t *>(o), nrm, mot, &depth);
+                std::memcpy(o + 1, nrm, 8); std::memcpy(o + 3, mot, 8); std::memcpy(o + 5, &depth, 4);
+                break;
+            }
+            case 3: o[0] = gbuffer_alpha_test(s, r.g, r.pid, r.u, r.v) ? 1u : 0u; break;
+            case 4:
+            case 5: {
+                RaytracedHit t = raytraced_hit(s, r.g, r.pid, r.u, r.v);
+                store_bgra8(reinterpret_cast<uint8_t *>(o), raytraced_color(pfd, kind == 5, t.albedo, t.N, false));
+                store_bgra8(reinterpret_cast<uint8_t *>(o + 1), raytraced_color(pfd, kind == 5, t.albedo, t.N, true));
+                std::memcpy(o + 2, &t.position, 12);
+                break;
+            }
+            case 6: o[0] = rahit_alpha_test(s, r.g, r.pid, r.u, r.v) ? 1u : 0u; break;
+        }
+    }
+    return 0;
 }
 
 // G-buffer scaffolding: primary rays through texel centres stand in for the rasteriser of the "G-Buffer Pass"
@@ -748,26 +895,11 @@ void vo_gbuffer(const vo_scene *s_, const PerFrameData *pfd_, int W, int H, uint
     for (int y = 0; y < H; ++y) {
         for (int x = 0; x < W; ++x) {
             size_t pix = (size_t)y * W + x;
-            vec2 uv = {((float)x + 0.5f) * pfd.display_size_inverse[0], ((float)y + 0.5f) * pfd.display_size_inverse[1]};
+            vec2 uv = gbuffer_pixel_uv(pfd, x, y);
             vec3 pn = get_world_space_position(pfd, 1.0f, uv);   // point on the near plane (reverse-Z: depth 1)
             vec3 dir = pn - cam;
             Hit h;
-            // gbuf.frag:19-32: fragments failing the alpha-mask test, or with alpha exactly 0, are discarded
-            auto alpha_test = [&](uint32_t tri, double hu, double hv) {
-                const Primitive &pr = s.primitives[s.tri_geom[tri]];
-                float alpha = pr.material.base_color[3];
-                if (has_texture(s, pr.material.base_color_texture)) {
-                    uint32_t k = s.tri_prim[tri];
-                    const Vertex &a0 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 0]];
-                    const Vertex &a1 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 1]];
-                    const Vertex &a2 = s.vertices[pr.vertex_offset + s.indices[pr.index_offset + 3 * k + 2]];
-                    float c1 = (float)hu, c2 = (float)hv, c0 = 1.0f - c1 - c2;
-                    vec2 uvt = {a0.uv0[0] * c0 + a1.uv0[0] * c1 + a2.uv0[0] * c2, a0.uv0[1] * c0 + a1.uv0[1] * c1 + a2.uv0[1] * c2};
-                    alpha = sample_texture(s, pr.material.base_color_texture, uvt).w;
-                }
-                if (pr.material.alpha_mask == 1 && alpha < pr.material.alpha_cutoff) return false;
-                return alpha != 0.0f;
-            };
+            auto alpha_test = [&](uint32_t tri, double hu, double hv) { return gbuffer_alpha_test(s, s.tri_geom[tri], s.tri_prim[tri], (float)hu, (float)hv); };
             bool hit = trace_closest_filtered(s, cam, dir, 1.0f, FLT_MAX, h, alpha_test);
             if (hit_ids) { hit_ids[2 * pix] = hit ? (int32_t)s.tri_geom[h.tri] : -1; hit_ids[2 * pix + 1] = hit ? (int32_t)s.tri_prim[h.tri] : -1; }
             if (!hit) {
@@ -777,65 +909,8 @@ void vo_gbuffer(const vo_scene *s_, const PerFrameData *pfd_, int W, int H, uint
                 depth[pix] = 0.0f;
                 continue;
             }
-            uint32_t g = s.tri_geom[h.tri], pid = s.tri_prim[h.tri];
-            const Primitive &prim = s.primitives[g];
-            const Vertex &v0 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
-            const Vertex &v1 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
-            const Vertex &v2 = s.vertices[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
-            float b1 = (float)h.u, b2 = (float)h.v, b0 = 1.0f - b1 - b2;
-            vec3 nobj = v3(v0.normal[0], v0.normal[1], v0.normal[2]) * b0 + v3(v1.normal[0], v1.normal[1], v1.normal[2]) * b1 +
-                        v3(v2.normal[0], v2.normal[1], v2.normal[2]) * b2;
-            vec3 pobj = v3(v0.pos[0], v0.pos[1], v0.pos[2]) * b0 + v3(v1.pos[0], v1.pos[1], v1.pos[2]) * b1 +
-                        v3(v2.pos[0], v2.pos[1], v2.pos[2]) * b2;
-            const Material &mat = prim.material;
-            vec2 tuv = {v0.uv0[0] * b0 + v1.uv0[0] * b1 + v2.uv0[0] * b2, v0.uv0[1] * b0 + v1.uv0[1] * b1 + v2.uv0[1] * b2};
-            vec4 albedo4 = {mat.base_color[0], mat.base_color[1], mat.base_color[2], mat.base_color[3]};
-            if (has_texture(s, mat.base_color_texture)) albedo4 = sample_texture(s, mat.base_color_texture, tuv);       // gbuf.frag:20-26
-            if (has_texture(s, mat.normal_map)) {                                                                     // gbuf.frag:35-41
-                vec4 c = sample_texture(s, mat.normal_map, tuv);
-                vec3 tsn = normalize(v3(c.x * 2.0f - 1.0f, c.y * 2.0f - 1.0f, c.z * 2.0f - 1.0f));
-                vec3 tan3 = v3(v0.tangent[0], v0.tangent[1], v0.tangent[2]) * b0 + v3(v1.tangent[0], v1.tangent[1], v1.tangent[2]) * b1 +
-                            v3(v2.tangent[0], v2.tangent[1], v2.tangent[2]) * b2;
-                float tw = v0.tangent[3] * b0 + v1.tangent[3] * b1 + v2.tangent[3] * b2;
-                vec3 bitangent = cross(tsn, tan3) * tw;
-                vec3 tangent = normalize(tan3 - nobj * dot(tan3, nobj));
-                nobj = tangent * tsn.x + bitangent * tsn.y + nobj * tsn.z;
-            }
-            float metallic = mat.metallic_factor, roughness = mat.roughness_factor;
-            if (has_texture(s, mat.metallic_roughness_texture)) {                                                     // gbuf.frag:52-56
-                vec4 c = sample_texture(s, mat.metallic_roughness_texture, tuv);
-                metallic *= c.y;
-                roughness *= c.z;
-            }
-            // normal_matrix = inverseTranspose(mat3(transform)) (hybrid_render_path.cpp:45) = cofactor(M) / det(M)
-            const float *m = prim.transform;
-            double a00 = m[0], a10 = m[1], a20 = m[2], a01 = m[4], a11 = m[5], a21 = m[6], a02 = m[8], a12 = m[9], a22 = m[10];
-            double c00 = a11 * a22 - a21 * a12, c01 = -(a10 * a22 - a20 * a12), c02 = a10 * a21 - a20 * a11;
-            double c10 = -(a01 * a22 - a21 * a02), c11 = a00 * a22 - a20 * a02, c12 = -(a00 * a21 - a20 * a01);
-            double c20 = a01 * a12 - a11 * a02, c21 = -(a00 * a12 - a10 * a02), c22 = a00 * a11 - a10 * a01;
-            double det = a00 * c00 + a01 * c01 + a02 * c02;
-            // (M^-T)[r][c] = cof[r][c] / det, with cof indexed [row][col] of M (a_rc = m[c*4+r])
-            float nm[9] = {(float)(c00 / det), (float)(c10 / det), (float)(c20 / det),    // column 0: rows 0..2
-                           (float)(c01 / det), (float)(c11 / det), (float)(c21 / det),    // column 1
-                           (float)(c02 / det), (float)(c12 / det), (float)(c22 / det)};   // column 2
-            vec3 nw = {nm[0] * nobj.x + nm[3] * nobj.y + nm[6] * nobj.z,
-                       nm[1] * nobj.x + nm[4] * nobj.y + nm[7] * nobj.z,
-                       nm[2] * nobj.x + nm[5] * nobj.y + nm[8] * nobj.z};
-            nw = normalize(nw);
-            vec4 pw = mul44(prim.transform, vec4{pobj.x, pobj.y, pobj.z, 1.0f});
-            vec4 clip = mul44(pfd.camera_proj, mul44(pfd.camera_view, pw));
-            vec4 pclip = mul44(pfd.camera_proj_prev_frame, mul44(pfd.camera_view_prev_frame, pw));
-            vec2 cur_ndc = uv;   // gl_FragCoord.xy * display_size_inverse
-            vec2 prev_ndc = {(pclip.x / pclip.w) * 0.5f + 0.5f, (pclip.y / pclip.w) * 0.5f + 0.5f};
-            if (albedo_bgra8) {
-                auto q = [](float f) { f = std::min(std::max(f, 0.0f), 1.0f); return (uint8_t)std::lrintf(f * 255.0f); };
-                albedo_bgra8[pix * 4 + 0] = q(albedo4.z); albedo_bgra8[pix * 4 + 1] = q(albedo4.y);
-                albedo_bgra8[pix * 4 + 2] = q(albedo4.x); albedo_bgra8[pix * 4 + 3] = q(albedo4.w);
-            }
-            store_rgba16f(normals, W, x, y, vec4{nw.x, nw.y, nw.z, (float)g});
-            store_rgba16f(motion, W, x, y, vec4{cur_ndc.x - prev_ndc.x, cur_ndc.y - prev_ndc.y,
-                                                metallic, roughness});
-            depth[pix] = clip.z / clip.w;
+            gbuffer_hit(s, pfd, s.tri_geom[h.tri], s.tri_prim[h.tri], (float)h.u, (float)h.v, uv, albedo_bgra8 ? albedo_bgra8 + pix * 4 : nullptr,
+                        normals + pix * 4, motion + pix * 4, depth + pix);
         }
     }
 }

@@ -63,7 +63,8 @@ def test_validation_context_tables_and_loud_failures():
         pc = np.zeros((), T.SVGFPushConstants)
         ctx.update_per_frame_ubo(np.zeros((), T.PerFrameData))
         for call in (lambda: ctx.dispatch("hybrid_render_path/svgf.comp", 8, 6, 1, pc), lambda: ctx.trace_rays(64, 48),
-                     lambda: ctx.image_upload("Depth", np.zeros((48, 64), np.float32))):
+                     lambda: ctx.image_upload("Depth", np.zeros((48, 64), np.float32)),
+                     lambda: ctx.shade_hits(T.SHADE_GBUFFER, np.zeros(2, T.ShadeRecord))):
             with pytest.raises(capi.VhrError) as e:
                 call()
             assert "VHR_DEVICE_NONE" in str(e.value)
@@ -74,6 +75,21 @@ def test_validation_context_tables_and_loud_failures():
                 ctx.upload_new_storage_image(8, 8, F4)
                 n += 1
         assert n == 2048 and "No free storage image slots" in str(e.value)
+
+
+def test_shade_hits_arguments_are_validated():
+    """vhr_debug_shade_hits: an unknown kind or a NULL array is VHR_ERR_INVALID before the device is needed; every kind fails loudly
+    on a validation-only context."""
+    with capi.Context(8, 8, device=host_api.DEVICE_NONE) as ctx:
+        rec = np.zeros(3, T.ShadeRecord)
+        for bad in (-1, T.SHADE_ANYHIT_ALPHA + 1, 1 << 20):
+            with pytest.raises(capi.VhrError, match="status -1:.*kind"):
+                ctx.shade_hits(bad, rec)
+        with pytest.raises(capi.VhrError, match="status -1:.*NULL"):
+            capi._check(capi.lib().vhr_debug_shade_hits(ctx._h, T.SHADE_TEXTURE, None, 3, capi._ptr(np.zeros(24, np.uint32))))
+        for kind in range(T.SHADE_ANYHIT_ALPHA + 1):
+            with pytest.raises(capi.VhrError, match="status -2:.*VHR_DEVICE_NONE"):
+                ctx.shade_hits(kind, rec)
 
 
 def test_per_frame_ubo_size_is_checked():

@@ -22,7 +22,7 @@ SYMBOLS = [
     "vhr_storage_image_device_ptr", "vhr_bind_pass_images", "vhr_dispatch", "vhr_trace_rays",
     "vhr_blit_storage_to_transient", "vhr_blit_transient_to_storage", "vhr_blit_storage_to_storage", "vhr_set_option",
     "vhr_get_option", "vhr_get_bvh_stats", "vhr_trace_explicit", "vhr_gbuffer_pass", "vhr_shadow_map_pass", "vhr_create_query_pool",
-    "vhr_write_timestamp", "vhr_get_query_elapsed_ms", "vhr_debug_download_reflection_t",
+    "vhr_write_timestamp", "vhr_get_query_elapsed_ms", "vhr_debug_download_reflection_t", "vhr_debug_shade_hits",
     "vhr_image_upload_async", "vhr_image_download_async", "vhr_wait_download", "vhr_draw",
     "vhr_set_partition", "vhr_image_export_ipc", "vhr_storage_image_export_ipc", "vhr_image_attach_peer",
     "vhr_storage_image_attach_peer", "vhr_sync_export_ipc", "vhr_sync_attach_peer",
@@ -140,6 +140,7 @@ def lib():
         L.vhr_sync_device_ptr.argtypes = [vp]
         L.vhr_sync_device_ptr.restype = vp
         L.vhr_debug_download_reflection_t.argtypes = [vp, vp, sz]
+        L.vhr_debug_shade_hits.argtypes = [vp, i32, vp, u32, vp]
         L.vhr_create_query_pool.argtypes = [vp, u32]
         L.vhr_write_timestamp.argtypes = [vp, u32]
         L.vhr_select_queue.argtypes = [vp, i32]
@@ -445,3 +446,11 @@ class Context:
         uv = np.empty((n, 2), np.float32)
         _check(lib().vhr_trace_explicit(self._h, _ptr(rays), n, int(bool(any_hit)), _ptr(t), _ptr(ids), _ptr(uv)))
         return t, ids, uv
+
+    def shade_hits(self, kind, records):
+        """vhr_debug_shade_hits: the per-hit shading of `kind` (types.SHADE_*) on the records (array of types.ShadeRecord).
+        Returns [n, types.SHADE_OUT_WORDS] uint32: the output words of each record (include/vhr_b200.h)."""
+        rec = np.ascontiguousarray(records, T.ShadeRecord).reshape(-1)
+        out = np.zeros((len(rec), T.SHADE_OUT_WORDS), np.uint32)
+        _check(lib().vhr_debug_shade_hits(self._h, int(kind), _ptr(rec), len(rec), _ptr(out)))
+        return out

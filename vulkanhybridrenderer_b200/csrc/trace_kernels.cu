@@ -6,12 +6,14 @@
 //   gbuffer_kernel  <- G-buffer encodings of gbuf.vert:19-28 / gbuf.frag:33,43,46-58 with primary rays standing in
 //                      for the rasteriser ("G-Buffer Pass", hybrid_render_path.cpp:13-56)
 //   trace_explicit  <- test/debug entry: explicit rays, any-hit or closest-hit
+//   shade_hits      <- test/debug entry: the per-hit shading of the passes on given (geometry, primitive, barycentrics)
 //
 // traceRayEXT semantics restated from the Vulkan ray-tracing spec (the reference's traversal lives in the driver):
 // opaque triangles, no culling (TLAS instance flag TRIANGLE_FACING_CULL_DISABLE, resource_manager.cpp:704-718),
 // a triangle counts when tMin < t < tMax, shared edges are watertight (Woop/Benthin/Wald 2013 with the double
 // fallback for zero edge functions).
 #include <stdlib.h>
+#include <string.h>
 
 #include <algorithm>
 #include <type_traits>
@@ -1107,59 +1109,19 @@ __device__ __forceinline__ float3 cross_rn(float3 a, float3 b) {
     return make_float3(sub_rn(mul_rn(a.y, b.z), mul_rn(a.z, b.y)), sub_rn(mul_rn(a.z, b.x), mul_rn(a.x, b.z)), sub_rn(mul_rn(a.x, b.y), mul_rn(a.y, b.x)));
 }
 
-// partitioned instance: the texel goes to the same place in every rank's image (of[rank] is this rank's own)
-template <typename T>
-__device__ __forceinline__ void store_every_rank(T *const *of, int world, size_t i, T v) {
-#pragma unroll
-    for (int r = 0; r < VHR_MAX_RANKS; ++r)
-        if (r < world) of[r][i] = v;
+// gl_FragCoord.xy * display_size_inverse of pixel (x, y)
+__device__ __forceinline__ float2 gbuffer_pixel_uv(const PerFrameData &pfd, int x, int y) {
+    return make_float2(mul_rn(add_rn((float)x, 0.5f), pfd.display_size_inverse[0]), mul_rn(add_rn((float)y, 0.5f), pfd.display_size_inverse[1]));
 }
 
-// PART = false: the single-GPU pass over the rows [y_begin, y_end). PART = true (GbufferPartParams): the rows dealt to this rank,
-// every texel stored to every rank; the per-pixel arithmetic is the same.
-template <bool PART>
-__global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ std::conditional_t<PART, GbufferPartParams, GbufferParams> p,
-                                                      const __grid_constant__ PerFrameData pfd) {
-    int x, y;
-    tile_coords(x, y);
-    if constexpr (PART) {
-        if (p.interleave)      // blockIdx.y counts this rank's 8-row blocks, dealt as raygen_kernel deals them
-            y = (y - blockIdx.y * 8) + (blockIdx.y * p.world + p.rank) * 8;
-        else
-            y += p.y_begin;
-    } else {
-        y += p.y_begin;
-    }
-    const bool in_range = x < p.W && y < p.y_end;       // trace() is warp-synchronous: no early return
-    const size_t pix = in_range ? (size_t)y * p.W + x : 0;
-    const float u = mul_rn(add_rn((float)x, 0.5f), pfd.display_size_inverse[0]);
-    const float v = mul_rn(add_rn((float)y, 0.5f), pfd.display_size_inverse[1]);
-    const float3 cam = make_float3(pfd.camera_view_inverse[12], pfd.camera_view_inverse[13], pfd.camera_view_inverse[14]);
-    const float3 pn = unproject_rn(pfd.camera_viewproj_inverse, 1.0f, u, v);   // near plane (reverse-Z: depth 1)
-    Ray ray;
-    ray.o = cam;
-    ray.d = make_float3(sub_rn(pn.x, cam.x), sub_rn(pn.y, cam.y), sub_rn(pn.z, cam.z));
-    ray.tmin = 1.0f;
-    ray.tmax = 3.0e38f;
-    Hit h;
-    const bool found = trace<false>(p.scene.nodes, p.scene.tris, p.scene.n_wide, p.scene.bias, ray, in_range, h, AlphaTest{p.scene});
-    if (!in_range) return;
-    if (!found) {
-        // clear values of hybrid_render_path.cpp:16-19
-        if constexpr (PART) {
-            store_every_rank(p.albedo_of, p.world, pix, 0u);
-            store_every_rank(p.normals_of, p.world, pix, make_uint2(0u, 0u));
-            store_every_rank(p.motion_of, p.world, pix, pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f)));
-            store_every_rank(p.depth_of, p.world, pix, 0.0f);
-        } else {
-            if (p.albedo) p.albedo[pix] = 0u;
-            p.normals[pix] = make_uint2(0u, 0u);
-            p.motion[pix] = pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f));
-            p.depth[pix] = 0.0f;
-        }
-        return;
-    }
-    const SceneRefs &s = p.scene;
+// The four words gbuf.frag stores for a primary hit of the pixel at (u, v) (gbuffer_pixel_uv): albedo BGRA8, normals / object id
+// RGBA16F, motion / metallic-roughness RGBA16F, depth D32.
+struct GbufferTexel {
+    uint32_t albedo;
+    uint2 normals, motion;
+    float depth;
+};
+__device__ __forceinline__ GbufferTexel gbuffer_hit(const SceneRefs &s, const PerFrameData &pfd, const Hit &h, float u, float v) {
     const float4 *tp = s.tris + (size_t)h.tri * 3;
     const uint32_t g = __float_as_uint(__ldg(tp).w), pid = __float_as_uint(__ldg(tp + 1).w);
     const Primitive &prim = s.prims[g];
@@ -1205,16 +1167,77 @@ __global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ st
     const float4 pclip = mul44_rn(pfd.camera_proj_prev_frame, mul44_rn(pfd.camera_view_prev_frame, pw));
     const float pu = add_rn(mul_rn(__fdiv_rn(pclip.x, pclip.w), 0.5f), 0.5f);
     const float pv = add_rn(mul_rn(__fdiv_rn(pclip.y, pclip.w), 0.5f), 0.5f);
+    GbufferTexel t;
+    t.albedo = unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24);
+    t.normals = pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g));
+    t.motion = pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness));
+    t.depth = __fdiv_rn(clip.z, clip.w);
+    return t;
+}
+
+// partitioned instance: the texel goes to the same place in every rank's image (of[rank] is this rank's own)
+template <typename T>
+__device__ __forceinline__ void store_every_rank(T *const *of, int world, size_t i, T v) {
+#pragma unroll
+    for (int r = 0; r < VHR_MAX_RANKS; ++r)
+        if (r < world) of[r][i] = v;
+}
+
+// PART = false: the single-GPU pass over the rows [y_begin, y_end). PART = true (GbufferPartParams): the rows dealt to this rank,
+// every texel stored to every rank; the per-pixel arithmetic is the same.
+template <bool PART>
+__global__ void __launch_bounds__(128) gbuffer_kernel(const __grid_constant__ std::conditional_t<PART, GbufferPartParams, GbufferParams> p,
+                                                      const __grid_constant__ PerFrameData pfd) {
+    int x, y;
+    tile_coords(x, y);
     if constexpr (PART) {
-        store_every_rank(p.albedo_of, p.world, pix, unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24));
-        store_every_rank(p.normals_of, p.world, pix, pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g)));
-        store_every_rank(p.motion_of, p.world, pix, pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness)));
-        store_every_rank(p.depth_of, p.world, pix, __fdiv_rn(clip.z, clip.w));
+        if (p.interleave)      // blockIdx.y counts this rank's 8-row blocks, dealt as raygen_kernel deals them
+            y = (y - blockIdx.y * 8) + (blockIdx.y * p.world + p.rank) * 8;
+        else
+            y += p.y_begin;
     } else {
-        if (p.albedo) p.albedo[pix] = unorm8(albedo.z) | (unorm8(albedo.y) << 8) | (unorm8(albedo.x) << 16) | (unorm8(albedo.w) << 24);
-        p.normals[pix] = pack_rgba16f(make_float4(nw.x, nw.y, nw.z, (float)g));
-        p.motion[pix] = pack_rgba16f(make_float4(sub_rn(u, pu), sub_rn(v, pv), metallic, roughness));
-        p.depth[pix] = __fdiv_rn(clip.z, clip.w);
+        y += p.y_begin;
+    }
+    const bool in_range = x < p.W && y < p.y_end;       // trace() is warp-synchronous: no early return
+    const size_t pix = in_range ? (size_t)y * p.W + x : 0;
+    const float2 puv = gbuffer_pixel_uv(pfd, x, y);
+    const float u = puv.x, v = puv.y;
+    const float3 cam = make_float3(pfd.camera_view_inverse[12], pfd.camera_view_inverse[13], pfd.camera_view_inverse[14]);
+    const float3 pn = unproject_rn(pfd.camera_viewproj_inverse, 1.0f, u, v);   // near plane (reverse-Z: depth 1)
+    Ray ray;
+    ray.o = cam;
+    ray.d = make_float3(sub_rn(pn.x, cam.x), sub_rn(pn.y, cam.y), sub_rn(pn.z, cam.z));
+    ray.tmin = 1.0f;
+    ray.tmax = 3.0e38f;
+    Hit h;
+    const bool found = trace<false>(p.scene.nodes, p.scene.tris, p.scene.n_wide, p.scene.bias, ray, in_range, h, AlphaTest{p.scene});
+    if (!in_range) return;
+    if (!found) {
+        // clear values of hybrid_render_path.cpp:16-19
+        if constexpr (PART) {
+            store_every_rank(p.albedo_of, p.world, pix, 0u);
+            store_every_rank(p.normals_of, p.world, pix, make_uint2(0u, 0u));
+            store_every_rank(p.motion_of, p.world, pix, pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f)));
+            store_every_rank(p.depth_of, p.world, pix, 0.0f);
+        } else {
+            if (p.albedo) p.albedo[pix] = 0u;
+            p.normals[pix] = make_uint2(0u, 0u);
+            p.motion[pix] = pack_rgba16f(make_float4(0.0f, 0.0f, -1.0f, -1.0f));
+            p.depth[pix] = 0.0f;
+        }
+        return;
+    }
+    const GbufferTexel t = gbuffer_hit(p.scene, pfd, h, u, v);
+    if constexpr (PART) {
+        store_every_rank(p.albedo_of, p.world, pix, t.albedo);
+        store_every_rank(p.normals_of, p.world, pix, t.normals);
+        store_every_rank(p.motion_of, p.world, pix, t.motion);
+        store_every_rank(p.depth_of, p.world, pix, t.depth);
+    } else {
+        if (p.albedo) p.albedo[pix] = t.albedo;
+        p.normals[pix] = t.normals;
+        p.motion[pix] = t.motion;
+        p.depth[pix] = t.depth;
     }
 }
 
@@ -1248,6 +1271,71 @@ struct RahitAlphaTest {
     }
 };
 
+// closesthit.rchit:11-41 for one hit: the albedo, the shading normal N and the world-space hit point (the shadow ray's origin)
+struct RaytracedHit {
+    float3 albedo, N, position;
+};
+__device__ __forceinline__ RaytracedHit raytraced_hit(const SceneRefs &s, const Hit &h) {
+    const float4 *tp = s.tris + (size_t)h.tri * 3;
+    const uint32_t g = __float_as_uint(__ldg(tp).w), pid = __float_as_uint(__ldg(tp + 1).w);
+    const Primitive &prim = s.prims[g];
+    const Vertex &v0 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
+    const Vertex &v1 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
+    const Vertex &v2 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
+    const float b1 = h.u, b2 = h.v, b0 = sub_rn(sub_rn(1.0f, b1), b2);
+    const float2 uv = bary_uv(v0, v1, v2, b0, b1, b2);
+    const float3 normal = bary3(f3(v0.normal), f3(v1.normal), f3(v2.normal), b0, b1, b2);
+    const float3 pobj = bary3(f3(v0.pos), f3(v1.pos), f3(v2.pos), b0, b1, b2);
+    const float4 pw = mul44_rn(prim.transform, make_float4(pobj.x, pobj.y, pobj.z, 1.0f));
+    RaytracedHit r;
+    r.albedo = make_float3(prim.material.base_color[0], prim.material.base_color[1], prim.material.base_color[2]);
+    if (has_texture(s, prim.material.base_color_texture)) {
+        const float4 c = sample_texture(s.textures, s.lut, prim.material.base_color_texture, uv.x, uv.y);
+        r.albedo = make_float3(c.x, c.y, c.z);
+    }
+    r.N = normal;
+    if (has_texture(s, prim.material.normal_map)) {
+        const float3 tan3 = bary3(f3(v0.tangent), f3(v1.tangent), f3(v2.tangent), b0, b1, b2);
+        const float tw = add_rn(add_rn(mul_rn(v0.tangent[3], b0), mul_rn(v1.tangent[3], b1)), mul_rn(v2.tangent[3], b2));
+        const float4 c = sample_texture(s.textures, s.lut, prim.material.normal_map, uv.x, uv.y);
+        const float3 tsn = normalize_rn(make_float3(sub_rn(mul_rn(c.x, 2.0f), 1.0f), sub_rn(mul_rn(c.y, 2.0f), 1.0f), sub_rn(mul_rn(c.z, 2.0f), 1.0f)));
+        const float3 cr = cross_rn(tsn, tan3);
+        const float3 bitangent = make_float3(mul_rn(cr.x, tw), mul_rn(cr.y, tw), mul_rn(cr.z, tw));
+        const float tdn = dot3_rn(tan3, normal);
+        const float3 tangent = normalize_rn(make_float3(sub_rn(tan3.x, mul_rn(normal.x, tdn)), sub_rn(tan3.y, mul_rn(normal.y, tdn)), sub_rn(tan3.z, mul_rn(normal.z, tdn))));
+        r.N = make_float3(add_rn(add_rn(mul_rn(tangent.x, tsn.x), mul_rn(bitangent.x, tsn.y)), mul_rn(normal.x, tsn.z)),
+                          add_rn(add_rn(mul_rn(tangent.y, tsn.x), mul_rn(bitangent.y, tsn.y)), mul_rn(normal.y, tsn.z)),
+                          add_rn(add_rn(mul_rn(tangent.z, tsn.x), mul_rn(bitangent.z, tsn.y)), mul_rn(normal.z, tsn.z)));
+    }
+    r.position = make_float3(pw.x, pw.y, pw.z);
+    return r;
+}
+
+// closesthit.rchit:43-57 / closesthit_test_alpha.rchit:37-50: the payload of a shaded hit given the shadow ray's answer
+template <bool ALPHA>
+__device__ __forceinline__ float4 raytraced_color(const PerFrameData &pfd, float3 albedo, float3 N, float3 L, bool occluded) {
+    const float amb = ALPHA ? 0.2f : VHR_PI_INVERSE;                                         // closesthit_test_alpha.rchit:39 / closesthit.rchit:46
+    float3 c = make_float3(mul_rn(amb, albedo.x), mul_rn(amb, albedo.y), mul_rn(amb, albedo.z));
+    if (!occluded) {
+        const float ndl = fmaxf(dot3_rn(N, L), 0.0f);
+        const float *li = pfd.directional_light.intensity, *lc = pfd.directional_light.color;
+        if (ALPHA) {
+            c = make_float3(add_rn(c.x, mul_rn(mul_rn(ndl, albedo.x), lc[0])), add_rn(c.y, mul_rn(mul_rn(ndl, albedo.y), lc[1])),
+                            add_rn(c.z, mul_rn(mul_rn(ndl, albedo.z), lc[2])));
+        } else {
+            c = make_float3(add_rn(c.x, mul_rn(mul_rn(mul_rn(ndl, albedo.x), li[0]), lc[0])), add_rn(c.y, mul_rn(mul_rn(mul_rn(ndl, albedo.y), li[1]), lc[1])),
+                            add_rn(c.z, mul_rn(mul_rn(mul_rn(ndl, albedo.z), li[2]), lc[2])));
+        }
+    }
+    return make_float4(c.x, c.y, c.z, 1.0f);
+}
+
+// imageStore to a B8G8R8A8_UNORM image: float -> UNORM8 (NaN -> 0), B in the low byte
+__device__ __forceinline__ uint32_t bgra8_word(float4 payload) {
+    auto q = [](float f) { f = (f == f) ? fminf(fmaxf(f, 0.0f), 1.0f) : 0.0f; return (uint32_t)__float2int_rn(f * 255.0f); };
+    return q(payload.z) | (q(payload.y) << 8) | (q(payload.x) << 16) | (q(payload.w) << 24);
+}
+
 template <bool ALPHA>
 __global__ void __launch_bounds__(128) raytraced_kernel(const __grid_constant__ RaytracedParams p, const __grid_constant__ PerFrameData pfd) {
     int x, y;
@@ -1277,37 +1365,10 @@ __global__ void __launch_bounds__(128) raytraced_kernel(const __grid_constant__ 
     const float3 L = make_float3(-pfd.directional_light.direction[0], -pfd.directional_light.direction[1], -pfd.directional_light.direction[2]);
     const bool shade = in_range && found;
     if (shade) {                                                                             // closesthit.rchit:11-41
-        const float4 *tp = s.tris + (size_t)h.tri * 3;
-        const uint32_t g = __float_as_uint(__ldg(tp).w), pid = __float_as_uint(__ldg(tp + 1).w);
-        const Primitive &prim = s.prims[g];
-        const Vertex &v0 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 0]];
-        const Vertex &v1 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 1]];
-        const Vertex &v2 = s.verts[prim.vertex_offset + s.indices[prim.index_offset + 3 * pid + 2]];
-        const float b1 = h.u, b2 = h.v, b0 = sub_rn(sub_rn(1.0f, b1), b2);
-        const float2 uv = bary_uv(v0, v1, v2, b0, b1, b2);
-        const float3 normal = bary3(f3(v0.normal), f3(v1.normal), f3(v2.normal), b0, b1, b2);
-        const float3 pobj = bary3(f3(v0.pos), f3(v1.pos), f3(v2.pos), b0, b1, b2);
-        const float4 pw = mul44_rn(prim.transform, make_float4(pobj.x, pobj.y, pobj.z, 1.0f));
-        albedo = make_float3(prim.material.base_color[0], prim.material.base_color[1], prim.material.base_color[2]);
-        if (has_texture(s, prim.material.base_color_texture)) {
-            const float4 c = sample_texture(s.textures, s.lut, prim.material.base_color_texture, uv.x, uv.y);
-            albedo = make_float3(c.x, c.y, c.z);
-        }
-        N = normal;
-        if (has_texture(s, prim.material.normal_map)) {
-            const float3 tan3 = bary3(f3(v0.tangent), f3(v1.tangent), f3(v2.tangent), b0, b1, b2);
-            const float tw = add_rn(add_rn(mul_rn(v0.tangent[3], b0), mul_rn(v1.tangent[3], b1)), mul_rn(v2.tangent[3], b2));
-            const float4 c = sample_texture(s.textures, s.lut, prim.material.normal_map, uv.x, uv.y);
-            const float3 tsn = normalize_rn(make_float3(sub_rn(mul_rn(c.x, 2.0f), 1.0f), sub_rn(mul_rn(c.y, 2.0f), 1.0f), sub_rn(mul_rn(c.z, 2.0f), 1.0f)));
-            const float3 cr = cross_rn(tsn, tan3);
-            const float3 bitangent = make_float3(mul_rn(cr.x, tw), mul_rn(cr.y, tw), mul_rn(cr.z, tw));
-            const float tdn = dot3_rn(tan3, normal);
-            const float3 tangent = normalize_rn(make_float3(sub_rn(tan3.x, mul_rn(normal.x, tdn)), sub_rn(tan3.y, mul_rn(normal.y, tdn)), sub_rn(tan3.z, mul_rn(normal.z, tdn))));
-            N = make_float3(add_rn(add_rn(mul_rn(tangent.x, tsn.x), mul_rn(bitangent.x, tsn.y)), mul_rn(normal.x, tsn.z)),
-                            add_rn(add_rn(mul_rn(tangent.y, tsn.x), mul_rn(bitangent.y, tsn.y)), mul_rn(normal.y, tsn.z)),
-                            add_rn(add_rn(mul_rn(tangent.z, tsn.x), mul_rn(bitangent.z, tsn.y)), mul_rn(normal.z, tsn.z)));
-        }
-        sray.o = make_float3(pw.x, pw.y, pw.z);
+        const RaytracedHit r = raytraced_hit(s, h);
+        albedo = r.albedo;
+        N = r.N;
+        sray.o = r.position;
         sray.d = L;
     }
     // closesthit.rchit:48-50: the shadow ray (miss index 1 clears shadow_payload). Every lane takes part; only shaded ones are alive.
@@ -1315,25 +1376,8 @@ __global__ void __launch_bounds__(128) raytraced_kernel(const __grid_constant__ 
     const bool occluded = ALPHA ? trace<true>(s.nodes, s.tris, s.n_wide, s.bias, sray, shade, sh, RahitAlphaTest{s})
                                 : trace<true>(s.nodes, s.tris, s.n_wide, s.bias, sray, shade, sh);
     if (!in_range) return;
-    if (shade) {
-        const float amb = ALPHA ? 0.2f : VHR_PI_INVERSE;                                     // closesthit_test_alpha.rchit:39 / closesthit.rchit:46
-        float3 c = make_float3(mul_rn(amb, albedo.x), mul_rn(amb, albedo.y), mul_rn(amb, albedo.z));
-        if (!occluded) {
-            const float ndl = fmaxf(dot3_rn(N, L), 0.0f);
-            const float *li = pfd.directional_light.intensity, *lc = pfd.directional_light.color;
-            if (ALPHA) {
-                c = make_float3(add_rn(c.x, mul_rn(mul_rn(ndl, albedo.x), lc[0])), add_rn(c.y, mul_rn(mul_rn(ndl, albedo.y), lc[1])),
-                                add_rn(c.z, mul_rn(mul_rn(ndl, albedo.z), lc[2])));
-            } else {
-                c = make_float3(add_rn(c.x, mul_rn(mul_rn(mul_rn(ndl, albedo.x), li[0]), lc[0])), add_rn(c.y, mul_rn(mul_rn(mul_rn(ndl, albedo.y), li[1]), lc[1])),
-                                add_rn(c.z, mul_rn(mul_rn(mul_rn(ndl, albedo.z), li[2]), lc[2])));
-            }
-        }
-        payload = make_float4(c.x, c.y, c.z, 1.0f);
-    }
-    // imageStore to a B8G8R8A8_UNORM image: float -> UNORM8 (NaN -> 0), B in the low byte
-    auto q = [](float f) { f = (f == f) ? fminf(fmaxf(f, 0.0f), 1.0f) : 0.0f; return (uint32_t)__float2int_rn(f * 255.0f); };
-    p.out[(size_t)y * p.W + x] = q(payload.z) | (q(payload.y) << 8) | (q(payload.x) << 16) | (q(payload.w) << 24);
+    if (shade) payload = raytraced_color<ALPHA>(pfd, albedo, N, L, occluded);
+    p.out[(size_t)y * p.W + x] = bgra8_word(payload);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1364,6 +1408,45 @@ __global__ void trace_explicit_kernel(const float *__restrict__ rays, uint32_t n
         out_ids[2 * i + 1] = found ? __float_as_uint(s.tris[(size_t)h.tri * 3 + 1].w) : 0xffffffffu;
     }
     if (out_uv) { out_uv[2 * i] = h.u; out_uv[2 * i + 1] = h.v; }
+}
+
+// vhr_debug_shade_hits (tests): record i's hit is triangle i of `s.tris`, a scratch array that carries only the record's (g, pid) in the
+// .w words the shading code reads, so the production per-hit code runs unchanged on hits chosen by the caller.
+__global__ void shade_hits_kernel(int kind, const vhr_shade_record *__restrict__ rec, uint32_t n, SceneRefs s,
+                                  const __grid_constant__ PerFrameData pfd, uint32_t *__restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const vhr_shade_record r = rec[i];
+    uint32_t *o = out + (size_t)VHR_SHADE_OUT_WORDS * i;
+    Hit h;
+    h.t = 0.0f; h.u = r.u; h.v = r.v; h.tri = i;
+    auto put4 = [&](float4 c) { o[0] = __float_as_uint(c.x); o[1] = __float_as_uint(c.y); o[2] = __float_as_uint(c.z); o[3] = __float_as_uint(c.w); };
+    switch (kind) {
+        case VHR_SHADE_TEXTURE: put4(sample_texture(s.textures, s.lut, (int)r.g, r.u, r.v)); break;
+        case VHR_SHADE_REFLECTION: put4(reflection_hit(s, pfd, h)); break;
+        case VHR_SHADE_GBUFFER: {
+            const float2 puv = gbuffer_pixel_uv(pfd, r.x, r.y);
+            const GbufferTexel t = gbuffer_hit(s, pfd, h, puv.x, puv.y);
+            o[0] = t.albedo; o[1] = t.normals.x; o[2] = t.normals.y; o[3] = t.motion.x; o[4] = t.motion.y; o[5] = __float_as_uint(t.depth);
+            break;
+        }
+        case VHR_SHADE_GBUFFER_ALPHA: o[0] = AlphaTest{s}(i, r.u, r.v) ? 1u : 0u; break;
+        case VHR_SHADE_RAYTRACED:
+        case VHR_SHADE_RAYTRACED_ALPHA: {
+            const RaytracedHit t = raytraced_hit(s, h);
+            const float3 L = make_float3(-pfd.directional_light.direction[0], -pfd.directional_light.direction[1], -pfd.directional_light.direction[2]);
+            if (kind == VHR_SHADE_RAYTRACED_ALPHA) {
+                o[0] = bgra8_word(raytraced_color<true>(pfd, t.albedo, t.N, L, false));
+                o[1] = bgra8_word(raytraced_color<true>(pfd, t.albedo, t.N, L, true));
+            } else {
+                o[0] = bgra8_word(raytraced_color<false>(pfd, t.albedo, t.N, L, false));
+                o[1] = bgra8_word(raytraced_color<false>(pfd, t.albedo, t.N, L, true));
+            }
+            o[2] = __float_as_uint(t.position.x); o[3] = __float_as_uint(t.position.y); o[4] = __float_as_uint(t.position.z);
+            break;
+        }
+        case VHR_SHADE_ANYHIT_ALPHA: o[0] = RahitAlphaTest{s}(i, r.u, r.v) ? 1u : 0u; break;
+    }
 }
 
 SceneRefs scene_refs(vhr_context *ctx) {
@@ -1612,6 +1695,34 @@ int launch_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int a
     if (out_uv) VHR_CUDA_CHECK(cudaMemcpyAsync(out_uv, d_uv, (size_t)n * 2 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
     cudaFree(d_rays); cudaFree(d_t); cudaFree(d_ids); cudaFree(d_uv);
+    return VHR_OK;
+}
+
+int launch_shade_hits(vhr_context *ctx, int kind, const vhr_shade_record *records, uint32_t n, uint32_t *out) {
+    if (n == 0) return VHR_OK;
+    const size_t out_bytes = (size_t)n * VHR_SHADE_OUT_WORDS * sizeof(uint32_t);
+    std::vector<float4> ids((size_t)n * 3, make_float4(0.0f, 0.0f, 0.0f, 0.0f));      // (g, pid) of record i in the .w of triangle i's first two rows
+    for (uint32_t i = 0; i < n; ++i) {
+        memcpy(&ids[(size_t)3 * i].w, &records[i].g, 4);
+        memcpy(&ids[(size_t)3 * i + 1].w, &records[i].pid, 4);
+    }
+    vhr_shade_record *d_rec = nullptr;
+    float4 *d_ids = nullptr;
+    uint32_t *d_out = nullptr;
+    VHR_CUDA_CHECK(cudaMalloc(&d_rec, (size_t)n * sizeof(vhr_shade_record)));
+    VHR_CUDA_CHECK(cudaMalloc(&d_ids, ids.size() * sizeof(float4)));
+    VHR_CUDA_CHECK(cudaMalloc(&d_out, out_bytes));
+    VHR_CUDA_CHECK(cudaMemcpyAsync(d_rec, records, (size_t)n * sizeof(vhr_shade_record), cudaMemcpyHostToDevice, ctx->stream));
+    VHR_CUDA_CHECK(cudaMemcpyAsync(d_ids, ids.data(), ids.size() * sizeof(float4), cudaMemcpyHostToDevice, ctx->stream));
+    VHR_CUDA_CHECK(cudaMemsetAsync(d_out, 0, out_bytes, ctx->stream));
+    SceneRefs s = scene_refs(ctx);
+    s.tris = d_ids;
+    shade_hits_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(kind, d_rec, n, s, ctx->pfd, d_out);
+    VHR_CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+    VHR_CUDA_CHECK(cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+    cudaFree(d_rec); cudaFree(d_ids); cudaFree(d_out);
     return VHR_OK;
 }
 

@@ -921,6 +921,29 @@ int vhr_debug_download_reflection_t(vhr_context *ctx, float *host, size_t bytes)
     return VHR_OK;
 }
 
+int vhr_debug_shade_hits(vhr_context *ctx, int kind, const vhr_shade_record *records, uint32_t n, uint32_t *out) {
+    if (!ctx || (n && (!records || !out))) return fail(VHR_ERR_INVALID, "NULL argument");
+    if (kind < VHR_SHADE_TEXTURE || kind > VHR_SHADE_ANYHIT_ALPHA) return fail(VHR_ERR_INVALID, "vhr_debug_shade_hits: kind %d", kind);
+    VHR_NEED_DEVICE(ctx);
+    if (!ctx->pfd_set) return fail(VHR_ERR_STATE, "vhr_update_per_frame_ubo has not been called");
+    VHR_CUDA_CHECK(cudaSetDevice(ctx->device));
+    if (kind == VHR_SHADE_TEXTURE) {
+        for (uint32_t i = 0; i < n; ++i)
+            if (records[i].g >= ctx->textures.size() || !ctx->textures[records[i].g].texels)
+                return fail(VHR_ERR_INVALID, "vhr_debug_shade_hits: record %u names texture slot %u, which holds no texture", i, records[i].g);
+    } else {
+        if (!ctx->d_primitives) return fail(VHR_ERR_STATE, "vhr_debug_shade_hits: no geometry (vhr_update_geometry)");
+        std::vector<Primitive> prims(ctx->n_primitives);
+        VHR_CUDA_CHECK(cudaMemcpyAsync(prims.data(), ctx->d_primitives, prims.size() * sizeof(Primitive), cudaMemcpyDeviceToHost, ctx->stream));
+        VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
+        for (uint32_t i = 0; i < n; ++i)
+            if (records[i].g >= ctx->n_primitives || records[i].pid >= prims[records[i].g].index_count / 3)
+                return fail(VHR_ERR_INVALID, "vhr_debug_shade_hits: record %u names triangle %u of geometry %u (%u geometries)", i, records[i].pid,
+                            records[i].g, ctx->n_primitives);
+    }
+    return launch_shade_hits(ctx, kind, records, n, out);
+}
+
 int vhr_get_bvh_stats(vhr_context *ctx, vhr_bvh_stats *out) {
     if (!ctx || !out) return fail(VHR_ERR_INVALID, "NULL argument");
     *out = ctx->bvh.stats;

@@ -191,6 +191,7 @@ int launch_shadow_map(vhr_context *ctx);        // shadow_map_kernels.cu
 void free_shadow_scratch(vhr_context *ctx);
 int launch_trace_explicit(vhr_context *ctx, const float *rays, uint32_t n, int any_hit, float *out_t, uint32_t *out_ids,
                           float *out_uv);
+int launch_shade_hits(vhr_context *ctx, int kind, const vhr_shade_record *records, uint32_t n, uint32_t *out);   // records validated
 // peer.cu: stream-ordered flag exchange with the other ranks (cuStreamWriteValue32 / cuStreamWaitValue32)
 int peer_sync_neighbours(vhr_context *ctx);   // after a kernel that pushed halo rows: tell both neighbours, wait for theirs
 int peer_sync_all(vhr_context *ctx);          // after the ray pass scattered its rows to their owners: all ranks <-> all ranks

@@ -57,6 +57,12 @@ Primitive = np.dtype([
     ("index_count", np.uint32),
 ])
 
+# vhr_shade_record (include/vhr_b200.h, vhr_debug_shade_hits): geometry index (texture kind: slot), primitive id, barycentrics of
+# vertices 1 and 2 (texture kind: s, t), pixel (G-buffer kind)
+ShadeRecord = np.dtype([("g", np.uint32), ("pid", np.uint32), ("u", np.float32), ("v", np.float32), ("x", np.int32), ("y", np.int32)])
+SHADE_TEXTURE, SHADE_REFLECTION, SHADE_GBUFFER, SHADE_GBUFFER_ALPHA, SHADE_RAYTRACED, SHADE_RAYTRACED_ALPHA, SHADE_ANYHIT_ALPHA = range(7)
+SHADE_OUT_WORDS = 8
+
 SVGFPushConstants = np.dtype([
     ("integrated_shadow_and_ao", np.int32, 2),
     ("prev_frame_normals_and_object_ids", np.int32),
