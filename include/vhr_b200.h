@@ -64,7 +64,8 @@ enum {
 int vhr_context_create(int device, void *cuda_stream, uint32_t width, uint32_t height, vhr_context **out);
 void vhr_context_destroy(vhr_context *ctx);
 const char *vhr_last_error(void);
-/* Blocks until everything enqueued on the context's stream has finished (reference: vkWaitForFences, renderer.cpp:107). */
+/* Blocks until everything enqueued on the context's stream has finished, a deferred a-trous dispatch included (vhr_dispatch)
+ * (reference: vkWaitForFences, renderer.cpp:107). */
 int vhr_context_synchronize(vhr_context *ctx);
 /* ComputeExecutionContext::GetDisplaySize (src/render_graph/compute_execution_context.cpp:8-10). */
 int vhr_get_display_size(vhr_context *ctx, uint32_t *width, uint32_t *height);
@@ -168,7 +169,15 @@ int vhr_bind_pass_images(vhr_context *ctx, const char *const *names_by_binding, 
  * SSRPushConstants (16 B, :41-46; bound images 0 albedo, 1 normals, 2 motion/metallic-roughness, 3 depth, 4 output) for SSR;
  * a size that does not match fails like the reference's assert (compute_execution_context.h:23).
  * The ssao.comp and ssr.comp dispatches first rewrite a scratch image of the library (16 bytes per texel of the depth image, one per
- * queue, allocated on first use): the 2 x 2 bilinear footprint of every depth texel, which their depth taps read with one load. */
+ * queue, allocated on first use): the 2 x 2 bilinear footprint of every depth texel, which their depth taps read with one load.
+ * A svgf_atrous_filter.comp dispatch is deferred: the kernel is launched, on the stream it was recorded for, when anything reads its
+ * output (a binding, the next SVGF dispatch, a blit source, a download, vhr_*_device_ptr), writes one of its images in place, frees
+ * an input, or calls vhr_context_synchronize, vhr_select_queue or vhr_set_partition; it is never launched if its output is overwritten
+ * whole before any read (the reference's last iteration, which the next frame's first iteration overwrites), its output image is
+ * destroyed, or the context is destroyed. Every image the caller can observe holds what the immediate launch would have left, and
+ * vhr_kernel_launch_count counts the kernel when it is launched. A device pointer exported before the dispatch shows its output only
+ * after one of the calls above has launched it. A timestamp (vhr_write_timestamp) written after such a dispatch can
+ * come before its kernel. Launches are immediate while a partition is installed, with VHR_OPT_SVGF_FUSED, and once queue 1 exists. */
 int vhr_dispatch(vhr_context *ctx, const char *shader_path, uint32_t x_groups, uint32_t y_groups, uint32_t z_groups,
                  const void *push_constants, size_t push_constants_size);
 

@@ -27,6 +27,8 @@ def main(W=1920, H=1080, reps=20):
     integ[..., 0] = rng.integers(0, 2, (H, W)); integ[..., 1] = rng.integers(0, 3, (H, W)) * 0.5
     integ[..., 2:] = rng.uniform(0, 0.25, (H, W, 2))
     with capi.Context(W, H) as ctx:
+        # with a second queue every a-trous dispatch launches at once: a deferred one would be dropped by the next dispatch's overwrite
+        ctx.select_queue(1); ctx.select_queue(0)
         ctx.update_per_frame_ubo(pfd)
         ctx.actualize_image("n", F4); ctx.image_upload("n", normals)
         a, b = ctx.upload_new_storage_image(W, H, F4), ctx.upload_new_storage_image(W, H, F4)

@@ -142,6 +142,7 @@ int vhr_set_partition(vhr_context *ctx, const vhr_partition *p) {
     // copy-free blits (VHR_OPT_BLIT_ALIAS) are suspended while a partition is installed — the peers hold mappings of fixed buffers — so every
     // image that still shares a buffer with a blit partner gets its own copy now
     if (ctx->device >= 0) {
+        if (int rc = launch_pending_atrous(ctx)) return rc;      // peers will store into these images unseen: no deferred dispatch
         for (auto &kv : ctx->transient)
             if (int rc = make_writable(ctx, &kv.second, false)) return rc;
         for (auto &im : ctx->storage)

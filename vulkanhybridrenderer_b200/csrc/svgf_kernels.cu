@@ -169,19 +169,8 @@ __global__ void __launch_bounds__(256, VHR_TEMPORAL_MIN_BLOCKS) svgf_temporal_ke
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// À-trous, variant 0: the reference's dataflow (one thread per pixel, direct loads)
+// À-trous, variant 0: the reference's dataflow (one thread per pixel, direct loads); AtrousParams: vhr_internal.h
 // ---------------------------------------------------------------------------------------------------------------
-struct AtrousParams {
-    int W, H;
-    int x_end, y_begin, y_end;
-    int step;
-    float dsx, dsy;
-    const uint2 *normals;      // binding 0
-    const uint2 *integ_in;     // storage_images[pc.integrated_shadow_and_ao[0]]
-    uint2 *integ_out;          // storage_images[pc.integrated_shadow_and_ao[1]]
-    HaloPush push;             // multi-GPU: boundary rows of the output also go to the neighbours' copies
-};
-
 __device__ __forceinline__ void store_out(const AtrousParams &p, int cy, size_t pix, uint2 v) {
     p.integ_out[pix] = v;
     if (p.push.rows) {
@@ -862,7 +851,7 @@ static EncodeTiledFn g_encode_tiled = nullptr;
 
 // (x, row mod S, row div S) view of a dense RGBA16F image, box = {box_w texels, 1, box_rows}. The image allocation is
 // padded by 16 rows of zeros (alloc_image), which is what the last partial slab (rows H .. ceil(H/S) S) reads.
-static int make_tensor_map(CUtensorMap *map, const Image *im, int S, int box_w, int box_rows) {
+static int make_tensor_map(CUtensorMap *map, const void *ptr, int width, int height, int S, int box_w, int box_rows) {
     if (!g_encode_tiled) {
         cudaDriverEntryPointQueryResult qres;
         void *fn = nullptr;
@@ -870,20 +859,20 @@ static int make_tensor_map(CUtensorMap *map, const Image *im, int S, int box_w, 
         if (!fn || qres != cudaDriverEntryPointSuccess) return fail(VHR_ERR_CUDA, "cuTensorMapEncodeTiled is not available in this driver");
         g_encode_tiled = (EncodeTiledFn)fn;
     }
-    const cuuint64_t W = im->width, H = im->height;
+    const cuuint64_t W = (cuuint64_t)width, H = (cuuint64_t)height;
     const cuuint64_t dims[3] = {W, (cuuint64_t)S, (H + S - 1) / S};
     const cuuint64_t strides[2] = {W * 8, W * 8 * (cuuint64_t)S};     // bytes, dims 1 and 2
     const cuuint32_t box[3] = {(cuuint32_t)box_w, 1u, (cuuint32_t)box_rows};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
-    CUresult r = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64 /* 8-byte elements: one texel */, 3, im->ptr, dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+    CUresult r = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64 /* 8-byte elements: one texel */, 3, const_cast<void *>(ptr), dims, strides, box,
+                                estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(VHR_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a %ux%u image, step %d", (int)r, im->width, im->height, S);
+    if (r != CUDA_SUCCESS) return fail(VHR_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a %dx%d image, step %d", (int)r, width, height, S);
     return VHR_OK;
 }
 
 template <int S, int PD, int RY, int TR>
-static int launch_tma(vhr_context *ctx, const AtrousParams &p, const Image *normals, const Image *in, int x_pixels, int y_pixels) {
+static int launch_tma(vhr_context *ctx, const AtrousParams &p, int x_pixels, int y_pixels) {
     typedef PairCfg<S, PD, RY, TR> C;
     typedef TmaCfg<S, PD, RY, TR> T;
     static_assert(T::SMEM <= 112 * 1024, "two CTAs per SM must fit in shared memory");
@@ -896,8 +885,8 @@ static int launch_tma(vhr_context *ctx, const AtrousParams &p, const Image *norm
     }
     const int sms = sms_of[ctx->device & 63];
     CUtensorMap map_n, map_i;
-    if (int rc = make_tensor_map(&map_n, normals, S, T::PCT, C::SR)) return rc;
-    if (int rc = make_tensor_map(&map_i, in, S, T::PCT, C::SR)) return rc;
+    if (int rc = make_tensor_map(&map_n, p.normals, p.W, p.H, S, T::PCT, C::SR)) return rc;
+    if (int rc = make_tensor_map(&map_i, p.integ_in, p.W, p.H, S, T::PCT, C::SR)) return rc;
     AtrousTmaParams q;
     q.a = p;
     q.n_tx = (x_pixels + 2 * PD - 1) / (2 * PD);
@@ -948,6 +937,8 @@ int launch_svgf_temporal(vhr_context *ctx, uint32_t xg, uint32_t yg, const SVGFP
         VHR_CUDA_CHECK(cudaMalloc(&mom->twin, mom->bytes));
         VHR_CUDA_CHECK(cudaMemsetAsync(mom->twin, 0, mom->bytes, ctx->stream));
     }
+    for (const Image *im : {prevn, hist, mom})
+        if ((rc = resolve_read(ctx, im))) return rc;
     if ((rc = make_writable(ctx, integ0, covers_image(ctx, integ0, (uint64_t)xg * 8, (uint64_t)yg * 8)))) return rc;
     TemporalParams p;
     p.W = (int)normals->width; p.H = (int)normals->height;
@@ -1000,6 +991,70 @@ int launch_svgf_temporal(vhr_context *ctx, uint32_t xg, uint32_t yg, const SVGFP
     return peer_sync_neighbours(ctx);
 }
 
+static int launch_direct(vhr_context *ctx, const AtrousParams &p, int x_pixels, int y_pixels) {
+    dim3 block(32, 8), grid((x_pixels + 31) / 32, (y_pixels + 7) / 8);
+    atrous_direct_kernel<<<grid, block, 0, ctx->stream>>>(p);
+    VHR_CUDA_CHECK(cudaGetLastError());
+    ctx->launches++;
+    return VHR_OK;
+}
+
+// The kernel instance of a dispatch: variant, step, and whether the UBO's display size matches the images
+static AtrousLauncher pick_launcher(const vhr_context *ctx, const AtrousParams &p) {
+    // The tiled kernel bounds-checks against the image size; the reference checks against pfd.display_size. They are
+    // the same thing whenever the UBO matches the images, which the tiled path requires.
+    bool tiled_ok = ctx->opt.atrous_variant >= 1 && p.dsx == (float)p.W && p.dsy == (float)p.H;
+    static const int dev_tr = getenv("VHR_ATROUS_TR") ? atoi(getenv("VHR_ATROUS_TR")) : 4;     // development A/B switch
+    if (tiled_ok && ctx->opt.atrous_variant >= 2 && dev_tr == 3) {      // three rows per thread, 192-thread CTAs (168 registers): 22 % fewer shared-memory loads per tap
+        switch (p.step) {
+            case 1: return launch_pair<1, 64, 3, 3>;
+            case 2: return launch_pair<2, 64, 3, 3>;
+            case 4: return launch_pair<4, 64, 3, 3>;
+            case 8: return launch_pair<8, 64, 3, 3>;
+            default: break;
+        }
+    }
+    if (tiled_ok && ctx->opt.atrous_variant >= 2 && dev_tr == 2) {
+        switch (p.step) {
+            case 1: return launch_pair<1, 64, 2, 2>;
+            case 2: return launch_pair<2, 64, 2, 2>;
+            case 4: return launch_pair<4, 64, 2, 2>;
+            case 8: return launch_pair<8, 64, 2, 2>;
+            case 16: return launch_pair<16, 64, 2, 2>;
+            default: break;
+        }
+    }
+    if (tiled_ok && ctx->opt.atrous_variant == 3 && (p.W % 2) == 0) {        // TMA needs 16-byte row strides
+        switch (p.step) {
+            case 1: return launch_tma<1, 64, 2, 4>;
+            case 2: return launch_tma<2, 64, 2, 4>;
+            case 4: return launch_tma<4, 64, 2, 4>;
+            case 8: return launch_tma<8, 64, 2, 4>;
+            default: break;   // step 16: the raw boxes no longer fit beside the planes twice per SM -> variant 2
+        }
+    }
+    if (tiled_ok && ctx->opt.atrous_variant >= 2) {
+        switch (p.step) {
+            case 1: return launch_pair<1, 64, 2, 4>;
+            case 2: return launch_pair<2, 64, 2, 4>;
+            case 4: return launch_pair<4, 64, 2, 4>;
+            case 8: return launch_pair<8, 64, 2, 4>;
+            case 16: return launch_pair<16, 64, 2, 4>;
+            default: break;   // other steps: direct kernel
+        }
+    } else if (tiled_ok) {
+        switch (p.step) {
+            case 1: return launch_tiled<1>;
+            case 2: return launch_tiled<2>;
+            case 4: return launch_tiled<4>;
+            case 8: return launch_tiled<8>;
+            case 16: return launch_tiled<16>;
+            default: break;   // other steps: direct kernel
+        }
+    }
+    return launch_direct;
+}
+
 static int atrous_launch_only(vhr_context *ctx, uint32_t xg, uint32_t yg, const SVGFPushConstants &pc, bool &pushed) {
     if (ctx->n_bound < 1) return fail(VHR_ERR_STATE, "svgf_atrous_filter.comp: pass images not bound");
     Image *normals = ctx->bound[0];
@@ -1011,7 +1066,10 @@ static int atrous_launch_only(vhr_context *ctx, uint32_t xg, uint32_t yg, const 
     if ((rc = check_image(out, VHR_FORMAT_R16G16B16A16_SFLOAT, normals, "atrous integrated[1]"))) return rc;
     if (in == out) return fail(VHR_ERR_INVALID, "atrous: integrated[0] and [1] are the same image");
     if (pc.atrous_step < 1) return fail(VHR_ERR_INVALID, "atrous: step %d < 1", pc.atrous_step);
+    if ((rc = resolve_read(ctx, in))) return rc;
     if ((rc = make_writable(ctx, out, covers_image(ctx, out, (uint64_t)xg * 8, (uint64_t)yg * 8)))) return rc;
+    // one deferred dispatch at a time: an earlier one that this dispatch did not read or overwrite whole goes first
+    if ((rc = launch_pending_atrous(ctx))) return rc;
     AtrousParams p;
     p.W = (int)normals->width; p.H = (int)normals->height;
     if (!dispatch_range(ctx, normals, xg, yg, p.x_end, p.y_begin, p.y_end)) return VHR_OK;
@@ -1023,67 +1081,60 @@ static int atrous_launch_only(vhr_context *ctx, uint32_t xg, uint32_t yg, const 
     if (ctx->part.enabled && p.step != ctx->part.no_exchange_step)
         p.push = halo_push_for(ctx, out, false, p.step == 1 ? std::max(4, ctx->part.motion_halo) : 4 * p.step);
     pushed = p.push.rows > 0;
-    // The tiled kernel bounds-checks against the image size; the reference checks against pfd.display_size. They are
-    // the same thing whenever the UBO matches the images, which the tiled path requires.
-    bool tiled_ok = ctx->opt.atrous_variant >= 1 && p.dsx == (float)p.W && p.dsy == (float)p.H;
-    static const int dev_tr = getenv("VHR_ATROUS_TR") ? atoi(getenv("VHR_ATROUS_TR")) : 4;     // development A/B switch
-    if (tiled_ok && ctx->opt.atrous_variant >= 2 && dev_tr == 3) {      // three rows per thread, 192-thread CTAs (168 registers): 22 % fewer shared-memory loads per tap
-        int xp = p.x_end, yp = p.y_end - p.y_begin;
-        switch (p.step) {
-            case 1: return launch_pair<1, 64, 3, 3>(ctx, p, xp, yp);
-            case 2: return launch_pair<2, 64, 3, 3>(ctx, p, xp, yp);
-            case 4: return launch_pair<4, 64, 3, 3>(ctx, p, xp, yp);
-            case 8: return launch_pair<8, 64, 3, 3>(ctx, p, xp, yp);
-            default: break;
-        }
-    }
-    if (tiled_ok && ctx->opt.atrous_variant >= 2 && dev_tr == 2) {
-        int xp = p.x_end, yp = p.y_end - p.y_begin;
-        switch (p.step) {
-            case 1: return launch_pair<1, 64, 2, 2>(ctx, p, xp, yp);
-            case 2: return launch_pair<2, 64, 2, 2>(ctx, p, xp, yp);
-            case 4: return launch_pair<4, 64, 2, 2>(ctx, p, xp, yp);
-            case 8: return launch_pair<8, 64, 2, 2>(ctx, p, xp, yp);
-            case 16: return launch_pair<16, 64, 2, 2>(ctx, p, xp, yp);
-            default: break;
-        }
-    }
-    if (tiled_ok && ctx->opt.atrous_variant == 3 && (p.W % 2) == 0) {        // TMA needs 16-byte row strides
-        int xp = p.x_end, yp = p.y_end - p.y_begin;
-        switch (p.step) {
-            case 1: return launch_tma<1, 64, 2, 4>(ctx, p, normals, in, xp, yp);
-            case 2: return launch_tma<2, 64, 2, 4>(ctx, p, normals, in, xp, yp);
-            case 4: return launch_tma<4, 64, 2, 4>(ctx, p, normals, in, xp, yp);
-            case 8: return launch_tma<8, 64, 2, 4>(ctx, p, normals, in, xp, yp);
-            default: break;   // step 16: the raw boxes no longer fit beside the planes twice per SM -> variant 2
-        }
-    }
-    if (tiled_ok && ctx->opt.atrous_variant >= 2) {
-        int xp = p.x_end, yp = p.y_end - p.y_begin;
-        switch (p.step) {
-            case 1: return launch_pair<1, 64, 2, 4>(ctx, p, xp, yp);
-            case 2: return launch_pair<2, 64, 2, 4>(ctx, p, xp, yp);
-            case 4: return launch_pair<4, 64, 2, 4>(ctx, p, xp, yp);
-            case 8: return launch_pair<8, 64, 2, 4>(ctx, p, xp, yp);
-            case 16: return launch_pair<16, 64, 2, 4>(ctx, p, xp, yp);
-            default: break;   // other steps: direct kernel
-        }
-    } else if (tiled_ok) {
-        int xp = p.x_end, yp = p.y_end - p.y_begin;
-        switch (p.step) {
-            case 1: return launch_tiled<1>(ctx, p, xp, yp);
-            case 2: return launch_tiled<2>(ctx, p, xp, yp);
-            case 4: return launch_tiled<4>(ctx, p, xp, yp);
-            case 8: return launch_tiled<8>(ctx, p, xp, yp);
-            case 16: return launch_tiled<16>(ctx, p, xp, yp);
-            default: break;   // other steps: direct kernel
-        }
-    }
-    dim3 block(32, 8), grid((p.x_end + 31) / 32, (p.y_end - p.y_begin + 7) / 8);
-    atrous_direct_kernel<<<grid, block, 0, ctx->stream>>>(p);
-    VHR_CUDA_CHECK(cudaGetLastError());
-    ctx->launches++;
+    const AtrousLauncher fn = pick_launcher(ctx, p);
+    const int xp = p.x_end, yp = p.y_end - p.y_begin;
+    // Deferred (PendingAtrous): the reference's last iteration writes an image that the next frame's iteration 0 overwrites unread
+    // (SURVEY Q1), so that launch is dropped; every other iteration is launched by the one after it, which reads its output.
+    if (ctx->part.enabled || ctx->opt.svgf_fused || ctx->queue[1]) return fn(ctx, p, xp, yp);
+    PendingAtrous &d = ctx->atrous_pending;
+    d.p = p; d.launch = fn; d.x_pixels = xp; d.y_pixels = yp; d.stream = ctx->stream;
+    d.valid = true;
     return VHR_OK;
+}
+
+int launch_pending_atrous(vhr_context *ctx) {
+    PendingAtrous &d = ctx->atrous_pending;
+    if (!d.valid) return VHR_OK;
+    d.valid = false;
+    VHR_CUDA_CHECK(cudaSetDevice(ctx->device));       // resolved from entry points that do not select the device themselves
+    cudaStream_t cur = ctx->stream;
+    ctx->stream = d.stream;
+    const int rc = d.launch(ctx, d.p, d.x_pixels, d.y_pixels);
+    ctx->stream = cur;
+    return rc;
+}
+
+int resolve_read(vhr_context *ctx, const Image *im) {
+    const PendingAtrous &d = ctx->atrous_pending;
+    return d.valid && im && im->ptr == d.p.integ_out ? launch_pending_atrous(ctx) : VHR_OK;
+}
+
+static bool recorded(const PendingAtrous &d, const void *buf) {
+    return buf && (buf == d.p.integ_out || buf == d.p.integ_in || buf == d.p.normals);
+}
+
+int resolve_touch(vhr_context *ctx, const Image *im) {
+    const PendingAtrous &d = ctx->atrous_pending;
+    return d.valid && im && recorded(d, im->ptr) ? launch_pending_atrous(ctx) : VHR_OK;
+}
+
+int resolve_free(vhr_context *ctx, const Image *im) {
+    PendingAtrous &d = ctx->atrous_pending;
+    if (d.valid && im && im->ptr == d.p.integ_out) {
+        d.valid = false;
+        return VHR_OK;
+    }
+    return resolve_touch(ctx, im);
+}
+
+int resolve_write(vhr_context *ctx, const void *buf, bool whole) {
+    PendingAtrous &d = ctx->atrous_pending;
+    if (!d.valid || !recorded(d, buf)) return VHR_OK;
+    if (whole && buf == d.p.integ_out) {
+        d.valid = false;
+        return VHR_OK;
+    }
+    return launch_pending_atrous(ctx);
 }
 
 int launch_svgf_atrous(vhr_context *ctx, uint32_t xg, uint32_t yg, const SVGFPushConstants &pc) {

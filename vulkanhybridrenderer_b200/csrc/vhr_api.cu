@@ -98,6 +98,7 @@ static int copy_out(vhr_context *ctx, Image *im, void *host, size_t bytes, const
     if (!im) return fail(VHR_ERR_INVALID, "%s: unknown image", what);
     if (!host || bytes != im->bytes) return fail(VHR_ERR_INVALID, "%s: %zu bytes given, image holds %zu", what, bytes, im->bytes);
     if (int rc = consume_upload(ctx, im)) return rc;
+    if (int rc = resolve_read(ctx, im)) return rc;
     VHR_CUDA_CHECK(cudaMemcpyAsync(host, im->ptr, bytes, cudaMemcpyDeviceToHost, ctx->stream));
     return VHR_OK;
 }
@@ -116,14 +117,17 @@ int vhr::make_writable(vhr_context *ctx, Image *im, bool whole) {
         VHR_CUDA_CHECK(cudaStreamWaitEvent(ctx->stream, im->direct_read_done, 0));
         im->direct_read_pending = false;
     }
-    if (!im || !im->shares_with) return VHR_OK;
+    if (!im) return VHR_OK;
+    if (!im->shares_with) return resolve_write(ctx, im->ptr, whole);
     Image *o = im->shares_with;
     void *sp = im->spare ? im->spare : o->spare;
     void *shared = im->ptr;
     im->ptr = sp;
     im->spare = o->spare = nullptr;
     im->shares_with = o->shares_with = nullptr;
-    // everything that read the idle allocation was enqueued before the blit that idled it, i.e. earlier on this stream
+    // `shared` stays with the partner, so a deferred a-trous dispatch that reads it keeps its input; a spare is never a buffer that
+    // dispatch recorded (blit() resolves it before it parks dst's buffer as the spare).
+    // Everything that read the idle allocation was enqueued before the blit that idled it, i.e. earlier on this stream
     if (!whole) VHR_CUDA_CHECK(cudaMemcpyAsync(im->ptr, shared, im->bytes, cudaMemcpyDeviceToDevice, ctx->stream));
     return VHR_OK;
 }
@@ -137,6 +141,7 @@ static int blit(vhr_context *ctx, Image *src, Image *dst, const char *what) {
                     src->height, src->format, dst->width, dst->height, dst->format);
     if (int rc = consume_upload(ctx, src)) return rc;
     if (int rc = consume_upload(ctx, dst)) return rc;
+    if (int rc = resolve_read(ctx, src)) return rc;
     if (src == dst || (dst->shares_with == src && dst->ptr == src->ptr)) return VHR_OK;      // already the same texels
     if (ctx->part.enabled && ctx->part.world > 1 && src->height == ctx->height) {
         if (int rc = make_writable(ctx, dst, false)) return rc;
@@ -217,6 +222,7 @@ void vhr_context_destroy(vhr_context *ctx) {
     if (!ctx) return;
     if (ctx->device < 0) { delete ctx; return; }
     cudaSetDevice(ctx->device);
+    // a deferred a-trous dispatch is dropped: nothing can read its output any more
     cudaStreamSynchronize(ctx->queue[0]);
     if (ctx->queue[1]) cudaStreamSynchronize(ctx->queue[1]);
     if (ctx->upload_stream) cudaStreamSynchronize(ctx->upload_stream);
@@ -251,6 +257,7 @@ void vhr_context_destroy(vhr_context *ctx) {
 int vhr_context_synchronize(vhr_context *ctx) {
     if (!ctx) return fail(VHR_ERR_INVALID, "ctx is NULL");
     if (ctx->device < 0) return VHR_OK;
+    if (int rc = launch_pending_atrous(ctx)) return rc;     // the GPU is idle with every recorded dispatch done on return
     VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->queue[0]));
     if (ctx->queue[1]) VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->queue[1]));
     if (ctx->upload_stream) VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->upload_stream));
@@ -264,6 +271,7 @@ int vhr_select_queue(vhr_context *ctx, int queue) {
     if (ctx->device < 0) return VHR_OK;      // validation-only context: nothing is recorded
     if (queue == 1 && ctx->part.enabled) return fail(VHR_ERR_STATE, "vhr_select_queue: not available while a partition is set (the peer flag words are ordered on queue 0)");
     VHR_CUDA_CHECK(cudaSetDevice(ctx->device));
+    if (int rc = launch_pending_atrous(ctx)) return rc;     // a-trous dispatches are not deferred once there is a second queue
     if (queue == 1 && !ctx->queue[1]) VHR_CUDA_CHECK(cudaStreamCreateWithFlags(&ctx->queue[1], cudaStreamNonBlocking));
     ctx->stream = ctx->queue[queue];
     return VHR_OK;
@@ -450,6 +458,7 @@ int vhr_destroy_storage_image(vhr_context *ctx, int slot) {
     if (!ctx) return fail(VHR_ERR_INVALID, "ctx is NULL");
     Image *im = storage_slot(ctx, slot);
     if (!im) return fail(VHR_ERR_INVALID, "storage image %d does not exist", slot);
+    if (int rc = resolve_free(ctx, im)) return rc;
     if (ctx->device >= 0) VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
     free_image(*im);
     return VHR_OK;
@@ -475,6 +484,8 @@ int vhr_actualize_image(vhr_context *ctx, const char *name, uint32_t width, uint
 
 int vhr_destroy_transient_resources(vhr_context *ctx) {
     if (!ctx) return fail(VHR_ERR_INVALID, "ctx is NULL");
+    for (auto &kv : ctx->transient)
+        if (int rc = resolve_free(ctx, &kv.second)) return rc;
     if (ctx->device >= 0) VHR_CUDA_CHECK(cudaStreamSynchronize(ctx->stream));
     for (auto &kv : ctx->transient) free_image(kv.second);
     ctx->transient.clear();
@@ -540,6 +551,7 @@ int vhr_image_download_async(vhr_context *ctx, const char *name, void *host, siz
     }
     // snapshot on the compute stream (a device-to-device copy at HBM speed), so later passes may overwrite the image
     // while the PCIe copy is still in flight; the snapshot itself is reused only after its previous read-back
+    if (int rc = resolve_read(ctx, im)) return rc;
     if (im->staging_busy) VHR_CUDA_CHECK(cudaStreamWaitEvent(ctx->stream, im->staging_free, 0));
     VHR_CUDA_CHECK(cudaMemcpyAsync(im->staging, im->ptr, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
     VHR_CUDA_CHECK(cudaEventRecord(im->staged, ctx->stream));
@@ -568,7 +580,7 @@ int vhr_wait_download(vhr_context *ctx, uint32_t ticket) {
 
 void *vhr_image_device_ptr(vhr_context *ctx, const char *name, uint32_t *width, uint32_t *height, int *vk_format) {
     Image *im = ctx ? find_transient(ctx, name) : nullptr;
-    if (!im) return nullptr;
+    if (!im || resolve_touch(ctx, im)) return nullptr;      // the caller may read or write through the pointer
     if (width) *width = im->width;
     if (height) *height = im->height;
     if (vk_format) *vk_format = im->format;
@@ -576,7 +588,7 @@ void *vhr_image_device_ptr(vhr_context *ctx, const char *name, uint32_t *width, 
 }
 void *vhr_storage_image_device_ptr(vhr_context *ctx, int slot, uint32_t *width, uint32_t *height, int *vk_format) {
     Image *im = ctx ? storage_slot(ctx, slot) : nullptr;
-    if (!im) return nullptr;
+    if (!im || resolve_touch(ctx, im)) return nullptr;      // the caller may read or write through the pointer
     if (width) *width = im->width;
     if (height) *height = im->height;
     if (vk_format) *vk_format = im->format;
@@ -590,8 +602,10 @@ int vhr_bind_pass_images(vhr_context *ctx, const char *const *names_by_binding, 
     for (uint32_t i = 0; i < count; ++i) {
         Image *im = names_by_binding ? find_transient(ctx, names_by_binding[i]) : nullptr;
         if (!im) return fail(VHR_ERR_INVALID, "binding %u: unknown image '%s'", i, (names_by_binding && names_by_binding[i]) ? names_by_binding[i] : "(null)");
-        if (ctx->device >= 0)
+        if (ctx->device >= 0) {
             if (int rc = consume_upload(ctx, im)) return rc;
+            if (int rc = resolve_read(ctx, im)) return rc;
+        }
         ctx->bound[i] = im;
     }
     ctx->n_bound = count;
@@ -803,6 +817,7 @@ int vhr_image_download_rows_async(vhr_context *ctx, const char *name, void *host
     VHR_CUDA_CHECK(cudaSetDevice(ctx->device));
     if (int rc = ensure_transfer_queues(ctx)) return rc;
     if (int rc = consume_upload(ctx, im)) return rc;
+    if (int rc = resolve_read(ctx, im)) return rc;
     const size_t row = im->bytes / im->height;
     VHR_CUDA_CHECK(cudaEventRecord(ctx->compute_tail, ctx->stream));
     VHR_CUDA_CHECK(cudaStreamWaitEvent(ctx->download_stream, ctx->compute_tail, 0));

@@ -102,6 +102,37 @@ struct HaloPush {
     int rows = 0;             // output rows [y_begin, y_begin+rows) go up, [y_end-rows, y_end) go down
 };
 
+// Kernel parameters of one a-trous dispatch (svgf_kernels.cu)
+struct AtrousParams {
+    int W, H;
+    int x_end, y_begin, y_end;
+    int step;
+    float dsx, dsy;
+    const uint2 *normals;      // binding 0
+    const uint2 *integ_in;     // storage_images[pc.integrated_shadow_and_ao[0]]
+    uint2 *integ_out;          // storage_images[pc.integrated_shadow_and_ao[1]]
+    HaloPush push;             // multi-GPU: boundary rows of the output also go to the neighbours' copies
+};
+typedef int (*AtrousLauncher)(vhr_context *ctx, const AtrousParams &p, int x_pixels, int y_pixels);
+
+// Deferred a-trous dispatch. launch_svgf_atrous records the launch instead of issuing it; it is resolved when something could observe
+// the difference, by buffer: the three buffers below are the ones the kernel reads and writes, as they were at record time.
+//   launched first: a read of `p.integ_out` (bind_pass_images, the SVGF dispatches' storage inputs, a blit source, every download),
+//                   a vhr_*_device_ptr export or a write of any of the three buffers (a write that make_writable moves to a fresh
+//                   allocation leaves the recorded buffer with the blit partner and needs nothing), the free of an input buffer,
+//                   vhr_context_synchronize, vhr_select_queue, vhr_set_partition, and the next a-trous dispatch;
+//   dropped:        a write that covers `p.integ_out` whole and does not read it (make_writable(..., whole = true) after the writer
+//                   resolved its reads), the free of `p.integ_out`, vhr_context_destroy.
+// Timestamps (vhr_write_timestamp) do not resolve it. Launches stay eager while a partition is installed (peers store into this rank's
+// images unseen), with VHR_OPT_SVGF_FUSED, and once a second queue exists.
+struct PendingAtrous {
+    bool valid = false;
+    AtrousParams p;
+    AtrousLauncher launch = nullptr;
+    int x_pixels = 0, y_pixels = 0;
+    cudaStream_t stream = nullptr;
+};
+
 }  // namespace vhr
 
 struct vhr_context {
@@ -145,6 +176,7 @@ struct vhr_context {
     // change an image, a binding or the per-frame constants: the note only holds for the very next such call.
     uint64_t epoch = 0;
     struct { bool valid = false; int in_slot = -1, out_slot = -1; uint64_t epoch = 0; } fused_it0;
+    vhr::PendingAtrous atrous_pending;             // see vhr::PendingAtrous
     std::vector<cudaEvent_t> queries;              // timestamp query pool
     // transfer queues: copies that overlap the compute stream (the reference's frames in flight, renderer.cpp:103-108)
     cudaStream_t upload_stream = nullptr, download_stream = nullptr;
@@ -197,9 +229,16 @@ int peer_sync_neighbours(vhr_context *ctx);   // after a kernel that pushed halo
 int peer_sync_all(vhr_context *ctx);          // after the ray pass scattered its rows to their owners: all ranks <-> all ranks
 HaloPush halo_push_for(vhr_context *ctx, Image *out, bool twin, int rows);
 void peer_close_all(vhr_context *ctx);
-// Call before enqueueing work that writes `im`: an image that shares its buffer with a blit partner gets the spare allocation
-// (its old content is copied over first unless the write covers the `whole` image). No-op for images that share nothing.
+// Call before enqueueing work that writes `im`, after resolving what that work reads (resolve_read): an image that shares its buffer
+// with a blit partner gets the spare allocation (its old content is copied over first unless the write covers the `whole` image); a
+// deferred a-trous dispatch that recorded the buffer written is launched first, or dropped if that buffer is its output and `whole`.
 int make_writable(vhr_context *ctx, Image *im, bool whole);
+// Deferred a-trous dispatch (PendingAtrous, svgf_kernels.cu)
+int launch_pending_atrous(vhr_context *ctx);              // launch it now, if there is one
+int resolve_read(vhr_context *ctx, const Image *im);      // `im` is about to be read: launch it if `im` holds its output
+int resolve_write(vhr_context *ctx, const void *buf, bool whole);   // `buf` is about to be written (make_writable)
+int resolve_touch(vhr_context *ctx, const Image *im);     // `im`'s buffer is handed out (device pointer export): launch it if it recorded that buffer
+int resolve_free(vhr_context *ctx, const Image *im);      // `im` is about to be freed: drop it if `im` holds its output, else resolve_touch
 // "'name'" of a transient image, "storage image <slot>" of a storage image (error messages)
 std::string image_label(vhr_context *ctx, const Image *im);
 // does a pass dispatched over xg x yg groups of 8 x 8 (or a w x h launch) overwrite every texel of `im`?
